@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DCLL hot path: RadioML IQ windows/sec (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one batch of synthetic IQ windows pushed through the whole hot path: IQ->spike encoding
 followed by T = 1024 timesteps of radio_ml_conv DCLL training (forward, local loss gradient, weight gradient
@@ -22,6 +22,11 @@ and Adam step per layer per timestep), or of inference for the infer workloads. 
                cores, on a bounded sample of the same workload; the oracle port when oracle/_ref is absent
 
 --impl reference times that CPU arm alone, on the same `config`.
+
+--dump-outputs DIR writes what the last timed step handed back to its caller -- the per-timestep class votes, every
+layer's parameters and, for training workloads, its neuron state -- as DIR/<name>.npy (float32), so that two builds run
+with the same arguments (hence the same seeded inputs) can be compared output for output.  Arrays larger than
+DUMP_SAMPLE elements are stored as a fixed seeded sample of DUMP_SAMPLE elements (<name>_sample.npy).
 """
 import argparse
 import json
@@ -50,6 +55,7 @@ WORKLOADS = {
 }
 DEFAULT = "radio_ml_conv_train_128x128_B64"
 K_CLASSES, N_IQ = 24, 1024
+DUMP_SAMPLE = 1 << 20          # elements kept per dumped array (4 MB): under 64 MB for every workload's arrays
 
 
 def peaks():
@@ -298,6 +304,41 @@ def build_net(wl, world=1):
     return net
 
 
+def sample_index(n):
+    """DUMP_SAMPLE sorted distinct indices into n > DUMP_SAMPLE elements, the same for every run: one index drawn from a
+    fixed seed inside each of DUMP_SAMPLE equal strata at the head of the flat array (its last n % DUMP_SAMPLE elements are
+    not sampled)."""
+    import numpy as np
+    stride = n // DUMP_SAMPLE
+    return np.arange(DUMP_SAMPLE) * stride + np.random.default_rng(0).integers(0, stride, DUMP_SAMPLE)
+
+
+def step_outputs(net, clout, train):
+    """{name: float32 array} of what a window hands back to its caller: the class votes clout [T, layers, B], and per layer
+    the parameters and, after a training window, the neuron state.  (Inference windows leave no state to compare: the
+    16x16 multi-timestep kernel keeps it on chip and returns only the votes.)  Arrays above DUMP_SAMPLE elements become
+    the sample at sample_index."""
+    import torch
+    arrays = {"clout": clout}
+    for i, sl in enumerate(net.dcll_slices):
+        lay = sl.dclllayer
+        arrays["l%d_weight" % i], arrays["l%d_bias" % i] = lay.i2h.weight, lay.i2h.bias
+        if lay.output_layer:
+            arrays["l%d_output_weight" % i], arrays["l%d_output_bias" % i] = lay.output_.weight, lay.output_.bias
+        if train:
+            for field, t in zip(lay.i2h.state._fields, lay.i2h.state):
+                arrays["l%d_%s" % (i, field)] = t
+    out, index = {}, {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            if t.numel() not in index:
+                index[t.numel()] = torch.from_numpy(sample_index(t.numel())).to(t.device)
+            t, name = t.reshape(-1)[index[t.numel()]], name + "_sample"
+        out[name] = t.float().cpu().numpy()
+    return out
+
+
 def _event_timed(fn, steps, flush=None):
     import torch
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -472,15 +513,16 @@ def run_b200(a):
     def run_window(cells, labels):
         net.reset()
         if not train:
-            net.test_window(cells)
-        elif world > 1:
-            net.learn_window_dp(cells, labels)
-        else:
-            net.learn_window(cells, labels)
+            return net.test_window(cells)
+        if world > 1:
+            return net.learn_window_dp(cells, labels)
+        return net.learn_window(cells, labels)
+
+    last = {}
 
     def step_device():
         cells, _ = iq2spiketrain(x_dev, y_dev, **enc)
-        run_window(cells, y_dev)
+        last["clout"] = run_window(cells, y_dev)
 
     def step_e2e():
         xd = x_pin.to("cuda", non_blocking=True)
@@ -519,6 +561,7 @@ def run_b200(a):
     launches = int(_lib.lib.dcll_launch_count(0))
     prof = _lib.profile_read()
     _lib.check(_lib.lib.dcll_profile_enable(0))
+    dumped = step_outputs(net, last["clout"], train) if a.dump_outputs and rank == 0 else None
     ms_e2e = timed(step_e2e, a.steps)
     clocks = sampler.stop() if sampler else None
     # BASELINE.json configs[4]: data-parallel training at GLOBAL batch 8192 (8192 / N windows per GPU; 16x16 script geometry, which
@@ -663,6 +706,10 @@ def run_b200(a):
         v, desc, spent, extra, kind = cpu_sample(a.workload, T, n_fwd=4 if big else 16, n_train=12 if big else 256)
         out["cpu_baseline"] = {"value": v, "unit": "windows/s", "cores": torch.get_num_threads(), "kind": kind,
                                "sample": desc, "seconds": spent, **extra}
+    if dumped is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     emit_json(out)
     if world > 1:
         dist.destroy_process_group()
@@ -716,7 +763,11 @@ def main():
                     help="fp32: FP32-exact parity mode on the FMA pipe; bf16x3: tcgen05, split-bf16 operands, 3 products per MAC; "
                          "f16x2 (headline mode): tcgen05, fp16 traces against split-fp16 weights / gradients, 2 products per MAC")
     ap.add_argument("--burnin", type=int, default=None, help="override the workload's burn-in (profiling runs)")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32; large arrays as a seeded sample)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to the B200 arm")
     if a.burnin is not None:
         w = list(WORKLOADS[a.workload])
         w[5] = a.burnin

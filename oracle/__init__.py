@@ -10,11 +10,12 @@ CPU fallback.
 
 Pinning: the reference ships no tests and no golden vectors (SURVEY.md section 4),
 so the oracle is pinned against outputs of the reference classes themselves,
-executed in the build container from /root/reference with four import shims
+executed from a checkout of the original project (BASELINE.json's
+reference_path, or DCLL_REFERENCE_ROOT) with four import shims
 (``oracle/refshim.py``).  The resulting fixtures live in ``tests/golden/`` next
 to the script that generated them (``tests/golden/make_golden.py``), and
 ``tests/test_oracle_vs_reference.py`` re-checks the oracle against the live
-reference whenever /root/reference is present.
+reference whenever that checkout or its vendored copy ``oracle/_ref`` is present.
 
 The quantised-weight path has NO counterpart in the reference ("parity
 unpinned", SURVEY.md section 8c); ``oracle/quant.py`` is the defining restatement.

@@ -1,5 +1,5 @@
-"""Import the UNMODIFIED reference on CPU: from /root/reference (build container) or from its vendored copy oracle/_ref/
-(written by oracle/make_ref.py; git-ignored, travels to the GPU box).
+"""Import the UNMODIFIED reference on CPU: from the checkout of the original project named by DCLL_REFERENCE_ROOT or by
+BASELINE.json's reference_path, else from its vendored copy oracle/_ref/ (written by oracle/make_ref.py; git-ignored).
 
 TEST / BASELINE INFRASTRUCTURE.  Used by ``tests/golden/make_golden.py`` (fixture generation),
 ``tests/test_oracle_vs_reference.py`` (skipped when no reference is present) and by ``bench.py``'s reference arm and
@@ -20,22 +20,22 @@ import os
 import sys
 import types
 
-VENDORED_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+from .make_ref import DST as VENDORED_ROOT, is_reference, source_candidates
 
 
 def _pick_root():
-    env = os.environ.get("DCLL_REFERENCE_ROOT")
-    for cand in ([env] if env else []) + ["/root/reference", VENDORED_ROOT]:
-        if cand and os.path.isfile(os.path.join(cand, "dcll", "pytorch_libdcll.py")):
+    cands = source_candidates()
+    for cand in cands + [VENDORED_ROOT]:
+        if is_reference(cand):
             return cand
-    return env or "/root/reference"
+    return cands[0] if cands else VENDORED_ROOT
 
 
 REFERENCE_ROOT = _pick_root()
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "dcll", "pytorch_libdcll.py"))
+    return is_reference(REFERENCE_ROOT)
 
 
 def _check_manifest(root):

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the live reference at /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs the original project (its checkout, see oracle/refshim.py, or oracle/_ref)")
 
 
 def pytest_collection_modifyitems(config, items):

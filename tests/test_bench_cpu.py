@@ -27,15 +27,19 @@ def test_reference_arm_runs_vendored_reference():
 
 
 def test_vendored_reference_manifest_guard(tmp_path):
-    """A modified vendored copy is refused (sha256 manifest)."""
-    import shutil
-    if not os.path.isfile(os.path.join(REF, "MANIFEST.json")):
-        pytest.skip("oracle/_ref not vendored")
-    dst = tmp_path / "_ref"
-    shutil.copytree(REF, dst)
+    """A modified vendored copy is refused (sha256 manifest).  The copy is vendored by make_ref from a stand-in source
+    tree: the guard reads the manifest before it imports anything."""
+    from oracle.make_ref import FILES, make_ref
+    src, dst = tmp_path / "src", tmp_path / "_ref"
+    for rel in FILES:
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_text("# %s\n" % rel)
+    assert make_ref(str(src), verbose=False, dst=str(dst))
+    code = "import os,sys; sys.path.insert(0, %r); os.environ['DCLL_REFERENCE_ROOT']=%r\nfrom oracle import refshim\nrefshim.load_reference()" % (ROOT, str(dst))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-2000:]
     with open(dst / "data" / "utils.py", "a") as f:
         f.write("\n# tampered\n")
-    code = "import os,sys; sys.path.insert(0, %r); os.environ['DCLL_REFERENCE_ROOT']=%r\nfrom oracle import refshim\nrefshim.load_reference()" % (ROOT, str(dst))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
     assert r.returncode != 0 and "sha256 mismatch" in r.stderr
 

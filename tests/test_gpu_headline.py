@@ -212,3 +212,33 @@ def test_tc_paths_with_conv_mma2_forced(mma2):
                         "-k", "forward_teacher_forced or weight_gradient or training_step or window_equals"],
                        cwd=root, env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
+
+
+def test_bench_dump_outputs_reproducible_and_steps_counted(tmp_path):
+    """bench.py --dump-outputs: two runs with the same arguments write the same float32 arrays (at most 64 MB); --steps sets
+    the number of timed windows (launches in the timed region scale with it, and one more window trains the weights on)."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(steps, d):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--workload",
+                            "radio_ml_conv_train_16x16_B64", "--timesteps", "64", "--steps", str(steps), "--warmup", "1",
+                            "--no-extras", "--no-cpu", "--dump-outputs", str(tmp_path / d)],
+                           cwd=root, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        return json.loads(r.stdout.strip().splitlines()[-1])
+
+    a, b, c = run(2, "a"), run(2, "b"), run(1, "c")
+    assert a["steps"] == 2 and a["gpu_launches"] == 2 * c["gpu_launches"] > 0
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) == sorted(os.listdir(tmp_path / "c")) and "clout.npy" in names
+    total = 0
+    for n in names:
+        x, y = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert x.dtype == np.float32 and np.array_equal(x, y), n
+        total += x.nbytes
+    assert total <= 64 << 20
+    assert np.load(tmp_path / "a" / "clout.npy").shape == (64, 3, 64)
+    assert not np.array_equal(np.load(tmp_path / "a" / "l2_weight.npy"), np.load(tmp_path / "c" / "l2_weight.npy"))

@@ -8,7 +8,6 @@ import pytest
 import torch
 
 from golden_util import NetFixture
-from oracle import refshim
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -74,18 +73,16 @@ def test_state_dict_keys_and_shapes_match_reference_fixture(cpu_modules, name):
     net.load_state_dict(fx.state_dict, strict=True)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not refshim.reference_available(), reason="reference not present")
-@pytest.mark.parametrize("spec,im_dims,K,arp", [("radio_ml_conv", (1, 16, 16), 24, 0.0), ("radio_ml_conv", (1, 16, 16), 24, 1.0),
-                                                 ("mnist_conv", (1, 28, 28), 10, 0.0)])
-def test_constructors_consume_rng_like_the_reference(cpu_modules, spec, im_dims, K, arp):
+@pytest.mark.parametrize("name", ["radio8_train", "radio8_arp_train", "mnist_train", "radioref_train"])
+def test_constructors_consume_rng_like_the_reference(cpu_modules, name):
     """Same seeds -> bit-identical initial parameters and time constants (torch + numpy RNG order:
-    reset_parameters -> nn.Linear inits -> reset_lc_parameters -> randomize_tau: tau_m then tau_s)."""
+    reset_parameters -> nn.Linear inits -> reset_lc_parameters -> randomize_tau: tau_m then tau_s).  The fixture holds the
+    state_dict of the reference's own ConvNetwork built at seed 1 (tests/golden/make_golden.py)."""
     L, N = cpu_modules
-    ref = refshim.build_reference_net(spec, im_dims, 4, K, arp=arp, seed=1)
-    net = _build(N, spec, im_dims, 4, K, arp)
+    fx = NetFixture(name)
+    net = _build(N, fx.spec_name, fx.im_dims, fx.B, fx.K, fx.arp)
     net.reset(True)
-    a, b = ref.state_dict(), net.state_dict()
+    a, b = fx.state_dict, net.state_dict()
     assert list(a.keys()) == list(b.keys())
     for k in a:
         assert torch.equal(a[k], b[k]), k

@@ -1,9 +1,9 @@
 """RadioML reader (SURVEY section 8f, row N4): host logic of data/load_radio_ml.py on an in-memory HDF5 stand-in.
 
 h5py and the 20 GB data set are not available, so the HDF5 module is replaced by a dictionary-backed fake with the four
-calls the reader makes (File, create_dataset, item access, close).  When /root/reference is present (build container) the
-reference's own RadioMLDataset runs on the SAME fake files and the two are compared element for element; everywhere the
-interleave / split / layout properties are checked directly.
+calls the reader makes (File, create_dataset, item access, close).  When the original project is present (oracle/refshim.py
+finds it), the reference's own RadioMLDataset runs on the SAME fake files and the two are compared element for
+element; everywhere the interleave / split / layout properties are checked directly.
 """
 import importlib.util
 import os
@@ -14,7 +14,9 @@ import numpy as np
 import pytest
 import torch
 
-REF = os.path.join(os.environ.get("DCLL_REFERENCE_ROOT", "/root/reference"), "data", "load_radio_ml.py")
+from oracle import refshim
+
+REF = os.path.join(refshim.REFERENCE_ROOT, "data", "load_radio_ml.py")
 
 
 class FakeH5:

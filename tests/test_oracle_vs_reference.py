@@ -1,9 +1,10 @@
-"""Pins the oracle against the LIVE reference (build container only; skipped on the GPU box).
+"""Pins the oracle against the LIVE reference (the checkout of the original project named by DCLL_REFERENCE_ROOT or
+BASELINE.json's reference_path, or its vendored copy oracle/_ref; skipped without one).
 
 The reference has no tests or golden vectors of its own (SURVEY.md section 4), so
 "the reference classes executed on the same inputs and seeds" is the definition
 of parity.  tests/golden/ holds the same comparisons frozen as fixtures so they
-also run where /root/reference is absent.
+also run where the reference is absent.
 """
 import copy
 
