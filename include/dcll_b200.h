@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define DCLL_ABI_VERSION 11
+#define DCLL_ABI_VERSION 12
 
 enum { DCLL_OK = 0, DCLL_EINVAL = -1, DCLL_ECUDA = -2, DCLL_EUNSUPPORTED = -3 };
 
@@ -34,9 +34,14 @@ enum { DCLL_COEF_SCALAR = 0, DCLL_COEF_CHANNEL = 1, DCLL_COEF_ELEMENT = 2 };
 /* layer input: dense float32 [B,Cin,H,W] spikes, or (layer 0 only, Cin == 1) the encoder's
  * int32 [B,2] (row, col) cell of the single spike of each sample. */
 enum { DCLL_X_DENSE = 0, DCLL_X_CELLS = 1 };
-/* loss classes train.py:173 can select; gradient of the mean-reduced loss. */
+/* loss classes train.py:173 can select (torch.nn.<class>() with default arguments); gradient of the mean-reduced loss.
+ * CROSS_ENTROPY: probability targets, softmax over the K values of a row, mean over the B rows; every other kind is
+ * element-wise, mean over the B*K elements.  BCE_LOGITS also serves MultiLabelSoftMarginLoss, SMOOTHL1 HuberLoss (delta 1);
+ * KL_DIV takes log-probability inputs, POISSON_NLL log-rate inputs; HINGE is HingeEmbeddingLoss (margin 1). */
 enum { DCLL_LOSS_SMOOTHL1 = 0, DCLL_LOSS_MSE = 1, DCLL_LOSS_L1 = 2,
-       DCLL_LOSS_EXTERNAL = 3 /* any other loss class: the host supplies dL/dpvoutput (and dL/doutput) */ };
+       DCLL_LOSS_EXTERNAL = 3 /* any other loss class: the host supplies dL/dpvoutput (and dL/doutput) */,
+       DCLL_LOSS_CROSS_ENTROPY = 4, DCLL_LOSS_BCE_LOGITS = 5, DCLL_LOSS_SOFT_MARGIN = 6, DCLL_LOSS_KL_DIV = 7,
+       DCLL_LOSS_POISSON_NLL = 8, DCLL_LOSS_HINGE = 9 /* the last kind */ };
 /* conv arithmetic: FP32 CUDA-core FMA (parity mode); split-bf16 x3 on tcgen05 tensor cores (both operands bf16 hi + lo, three
  * products); or F16X2: the same kernels with the TRACE operand as one fp16 value (eps1 lies in [0,1]: relative rounding 2^-12)
  * against split-fp16 weights / local gradients -- two products, no lo pass over the traces.  kind::f16 wants both operands in

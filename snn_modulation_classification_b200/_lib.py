@@ -8,12 +8,13 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libdcll_b200.so")
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 OK, EINVAL, ECUDA, EUNSUPPORTED = 0, -1, -2, -3
 COEF_SCALAR, COEF_CHANNEL, COEF_ELEMENT = 0, 1, 2
 X_DENSE, X_CELLS = 0, 1
 LOSS_SMOOTHL1, LOSS_MSE, LOSS_L1, LOSS_EXTERNAL = 0, 1, 2, 3
+LOSS_CROSS_ENTROPY, LOSS_BCE_LOGITS, LOSS_SOFT_MARGIN, LOSS_KL_DIV, LOSS_POISSON_NLL, LOSS_HINGE = 4, 5, 6, 7, 8, 9
 PREC_FP32, PREC_BF16X3, PREC_F16X2 = 0, 1, 2
 
 _fp = C.c_void_p  # device pointers travel as integers

@@ -262,18 +262,58 @@ __device__ __forceinline__ float sigmoidf_ref(float x) {
     return __fdiv_rn(1.f, __fadd_rn(1.f, expf(-x)));
 }
 
-// d(mean-reduced loss)/d(pred): torch multiplies by norm = float(1/numel) (float(2/numel) for MSE),
+// Element-wise losses of a read-out value x against its target y (every kind except DCLL_LOSS_CROSS_ENTROPY).
+// d(mean-reduced loss)/dx: torch multiplies by norm = float(1/numel) (float(2/numel) for MSE),
 // aten/src/ATen/native/cpu/PointwiseOpsKernel.cpp (smooth_l1_backward, mse_backward).
-__device__ __forceinline__ float loss_grad_elem(float d, int kind, int numel) {
+__device__ __forceinline__ float loss_grad_elem(float x, float y, int kind, int numel) {
+    const float d = x - y;
     if (kind == DCLL_LOSS_MSE) return __fmul_rn((float)(2.0 / (double)numel), d);
     const float norm = (float)(1.0 / (double)numel);
     if (kind == DCLL_LOSS_SMOOTHL1) return d < -1.f ? -norm : (d > 1.f ? norm : __fmul_rn(norm, d));
-    return d > 0.f ? norm : (d < 0.f ? -norm : 0.f);
+    if (kind == DCLL_LOSS_L1) return d > 0.f ? norm : (d < 0.f ? -norm : 0.f);
+    if (kind == DCLL_LOSS_BCE_LOGITS) return __fmul_rn(__fsub_rn(sigmoidf_ref(x), y), norm);
+    if (kind == DCLL_LOSS_SOFT_MARGIN) return __fmul_rn(__fmul_rn(-y, sigmoidf_ref(-y * x)), norm);
+    if (kind == DCLL_LOSS_KL_DIV) return __fmul_rn(-y, norm);
+    if (kind == DCLL_LOSS_POISSON_NLL) return __fmul_rn(__fsub_rn(expf(x), y), norm);
+    // DCLL_LOSS_HINGE, torch's form for any target: where(y != 1, clamp_min(1 - x, 0), 0) + where(y != -1, x, 0); the
+    // clamp passes its gradient at 1 - x == 0, so for y = 0 the slope at x = 1 is -1 + 1 = 0
+    return ((y != -1.f) ? norm : 0.f) - ((y != 1.f && x <= 1.f) ? norm : 0.f);
 }
-__device__ __forceinline__ float loss_value_elem(float d, int kind) {
+// loss of one element before the 1/numel of the mean
+__device__ __forceinline__ float loss_value_elem(float x, float y, int kind) {
+    const float d = x - y;
     if (kind == DCLL_LOSS_SMOOTHL1) return fabsf(d) < 1.f ? 0.5f * d * d : fabsf(d) - 0.5f;
     if (kind == DCLL_LOSS_MSE) return d * d;
-    return fabsf(d);
+    if (kind == DCLL_LOSS_L1) return fabsf(d);
+    if (kind == DCLL_LOSS_BCE_LOGITS) return fmaxf(x, 0.f) - y * x + log1pf(expf(-fabsf(x)));      // softplus(x) - y x
+    if (kind == DCLL_LOSS_SOFT_MARGIN) {                                                            // softplus(-y x)
+        const float z = -y * x;
+        return fmaxf(z, 0.f) + log1pf(expf(-fabsf(z)));
+    }
+    if (kind == DCLL_LOSS_KL_DIV) return (y == 0.f ? 0.f : y * logf(y)) - y * x;                  // xlogy(y, y) - y x
+    if (kind == DCLL_LOSS_POISSON_NLL) return expf(x) - y * x;
+    return ((y != 1.f) ? fmaxf(1.f - x, 0.f) : 0.f) + ((y != -1.f) ? x : 0.f);                     // DCLL_LOSS_HINGE
+}
+
+// torch.nn.CrossEntropyLoss() with probability targets, mean over the B rows, for element k of one row x[0..K) with target
+// row y: returns g_k = (softmax(x)_k * sum(y) - y_k) / B (torch's gradient also for rows that do not sum to 1) and adds
+// -y_k log_softmax(x)_k / B to `val`.  The row maximum is subtracted before expf, so every finite row stays finite.
+// Every caller of a row walks it whole, in the same fixed order (maximum, then the sums over k = 0..K-1): one CTA per row
+// in readout_finish_kernel, one thread per element in loss_grad_kernel and dense_loss_grad_kernel all get the same bits
+// from the same row values.
+__device__ __forceinline__ float ce_grad_elem(const float *x, const float *y, int K, int k, int B, float &val) {
+    float m = x[0];
+    for (int j = 1; j < K; ++j) m = fmaxf(m, x[j]);
+    float s = 0.f, ysum = 0.f;
+    for (int j = 0; j < K; ++j) {
+        s = __fadd_rn(s, expf(__fsub_rn(x[j], m)));
+        ysum = __fadd_rn(ysum, y[j]);
+    }
+    const float inv_b = (float)(1.0 / (double)B);
+    const float xk = __fsub_rn(x[k], m), yk = y[k];
+    val += __fmul_rn(__fmul_rn(-yk, __fsub_rn(xk, logf(s))), inv_b);
+    const float p = __fdiv_rn(expf(xk), s);
+    return __fmul_rn(__fsub_rn(__fmul_rn(p, ysum), yk), inv_b);
 }
 
 }  // namespace dcll

@@ -109,11 +109,18 @@ __global__ void dense_finish_kernel(const float *__restrict__ pvoutput, int B, i
     clout[b] = best;
 }
 
-__global__ void dense_loss_grad_kernel(const float *__restrict__ pvoutput, const float *__restrict__ target, int n,
+__global__ void dense_loss_grad_kernel(const float *__restrict__ pvoutput, const float *__restrict__ target, int B, int K,
                                        int loss_kind, float *__restrict__ g_o) {
     pdl_entry();
     int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) g_o[i] = loss_grad_elem(pvoutput[i] - target[i], loss_kind, n);
+    if (i >= B * K) return;
+    if (loss_kind == DCLL_LOSS_CROSS_ENTROPY) {
+        const int b = i / K;
+        float unused = 0.f;   // the host computes the dense loss value itself
+        g_o[i] = ce_grad_elem(pvoutput + (size_t)b * K, target + (size_t)b * K, K, i - b * K, B, unused);
+    } else {
+        g_o[i] = loss_grad_elem(pvoutput[i], target[i], loss_kind, B * K);
+    }
 }
 
 __global__ void colsum_kernel(const float *__restrict__ g, int B, int N, float *__restrict__ out) {
@@ -179,12 +186,14 @@ extern "C" __attribute__((visibility("default"))) int dcll_dense_step_bwd_update
     DCLL_REQUIRE(a && L->g_o && L->g_u && L->grad_w && L->grad_b, DCLL_EINVAL, "dcll_dense_step_bwd_update: null scratch");
     cudaStream_t st = (cudaStream_t)stream;
     const int nk = L->B * L->K;
+    DCLL_REQUIRE(a->loss_kind >= DCLL_LOSS_SMOOTHL1 && a->loss_kind <= DCLL_LOSS_HINGE, DCLL_EINVAL,
+                 "dcll_dense_step_bwd_update: unknown loss");
     if (a->loss_kind == DCLL_LOSS_EXTERNAL) {
         DCLL_REQUIRE(a->g_o_ext, DCLL_EINVAL, "dcll_dense_step_bwd_update: external loss gradient missing");
         DCLL_CUDA_OK(cudaMemcpyAsync(L->g_o, a->g_o_ext, sizeof(float) * nk, cudaMemcpyDeviceToDevice, st));
     } else {
         DCLL_REQUIRE(a->target, DCLL_EINVAL, "dcll_dense_step_bwd_update: null target");
-        launch_k(dense_loss_grad_kernel, ceil_div(nk, 256), 256, 0, st, L->pvoutput, a->target, nk, a->loss_kind, L->g_o);
+        launch_k(dense_loss_grad_kernel, ceil_div(nk, 256), 256, 0, st, L->pvoutput, a->target, L->B, L->K, a->loss_kind, L->g_o);
         DCLL_LAUNCH_OK("dense_loss_grad_kernel");
     }
     GemmP p = {};                                      // g_u[b,o] = (sum_k g_o[b,k] Wo[k,o]) * pv (1-pv)

@@ -192,7 +192,7 @@ static int step_bwd(dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st) {
 static int check_train(const dcll_conv_layer *L, const dcll_train_args *a, const char *who) {
     DCLL_REQUIRE(a, DCLL_EINVAL, "%s: null train args", who);
     DCLL_REQUIRE(L->g_u, DCLL_EINVAL, "%s: null g_u scratch", who);
-    DCLL_REQUIRE(a->loss_kind >= DCLL_LOSS_SMOOTHL1 && a->loss_kind <= DCLL_LOSS_EXTERNAL, DCLL_EINVAL, "%s: unknown loss", who);
+    DCLL_REQUIRE(a->loss_kind >= DCLL_LOSS_SMOOTHL1 && a->loss_kind <= DCLL_LOSS_HINGE, DCLL_EINVAL, "%s: unknown loss", who);
     DCLL_REQUIRE(a->loss_kind != DCLL_LOSS_EXTERNAL || (a->g_o_ext && (!L->output_layer || a->g_o2_ext)), DCLL_EINVAL,
                  "%s: external loss gradient missing", who);
     if (a->apply_update) {

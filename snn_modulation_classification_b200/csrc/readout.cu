@@ -181,14 +181,20 @@ __global__ void __launch_bounds__(1024) readout_finish_kernel(const float *__res
         v += second ? bout[k] : bo[k];
         vals[tid] = v;
         (second ? output : pvoutput)[(size_t)b * K + k] = v;
-        if (target) {
-            float d = v - target[(size_t)b * K + k];
-            float g = loss_grad_elem(d, loss_kind, B * K);
+        if (target && loss_kind != DCLL_LOSS_CROSS_ENTROPY) {
+            const float y = target[(size_t)b * K + k];
+            float g = loss_grad_elem(v, y, loss_kind, B * K);
             (second ? g_o2 : g_o)[(size_t)b * K + k] = g;
-            lsum = loss_value_elem(d, loss_kind) / (float)(B * K);
+            lsum = loss_value_elem(v, y, loss_kind) / (float)(B * K);
         }
     }
     __syncthreads();
+    if (target && loss_kind == DCLL_LOSS_CROSS_ENTROPY && tid < Ktot) {
+        // row-coupled: each head (pvoutput, output) gets its own softmax over the K values now in `vals`
+        const bool second = tid >= K;
+        const int k = second ? tid - K : tid;
+        (second ? g_o2 : g_o)[(size_t)b * K + k] = ce_grad_elem(vals + (second ? K : 0), target + (size_t)b * K, K, k, B, lsum);
+    }
     if (tid == 0) {
         // DCLLClassification.forward :725-728 -- argmax of output on the output layer, else of pvoutput;
         // first maximum wins, as torch.argmax does.
@@ -744,22 +750,26 @@ __global__ void __launch_bounds__(256, 3) wout_grad_adam2_kernel(const float *__
     }
 }
 
-// g_o / g_o2 from stored read-outs (layer-level API: the target is only known after forward returned)
+// g_o / g_o2 from stored read-outs (layer-level API: the target is only known after forward returned).  One thread per
+// element; with cross-entropy each thread walks its row (K <= 32, rows stay in L1) exactly as readout_finish_kernel does.
 __global__ void loss_grad_kernel(const float *__restrict__ pvoutput, const float *__restrict__ output,
                                  const float *__restrict__ target, int B, int K, int loss_kind, float *__restrict__ g_o,
                                  float *__restrict__ g_o2, float *__restrict__ loss_out) {
     pdl_entry();
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     float lsum = 0.f;
-    if (i < B * K) {
+    if (i < B * K && loss_kind == DCLL_LOSS_CROSS_ENTROPY) {
+        const int b = i / K, k = i - b * K;
+        const float *y = target + (size_t)b * K;
+        g_o[i] = ce_grad_elem(pvoutput + (size_t)b * K, y, K, k, B, lsum);
+        if (output) g_o2[i] = ce_grad_elem(output + (size_t)b * K, y, K, k, B, lsum);
+    } else if (i < B * K) {
         float t = target[i];
-        float d = pvoutput[i] - t;
-        g_o[i] = loss_grad_elem(d, loss_kind, B * K);
-        lsum = loss_value_elem(d, loss_kind) / (float)(B * K);
+        g_o[i] = loss_grad_elem(pvoutput[i], t, loss_kind, B * K);
+        lsum = loss_value_elem(pvoutput[i], t, loss_kind) / (float)(B * K);
         if (output) {
-            float d2 = output[i] - t;
-            g_o2[i] = loss_grad_elem(d2, loss_kind, B * K);
-            lsum += loss_value_elem(d2, loss_kind) / (float)(B * K);
+            g_o2[i] = loss_grad_elem(output[i], t, loss_kind, B * K);
+            lsum += loss_value_elem(output[i], t, loss_kind) / (float)(B * K);
         }
     }
     if (loss_out) {

@@ -608,9 +608,11 @@ class Conv2dDCLLlayer(nn.Module):
         return old, outs
 
     def _grad_exp(self, batch):
-        """Exponent of the g_u image ('f16x2'): |g_u| <= sum_k |g_o| |Wo| / 4 <= max|Wo| / (4 B) for the mean-reduced SmoothL1 /
-        L1 losses (|g_o| <= 1/(B K)); 2^4 of slack for MSE residuals above 1 and external losses, the store saturates beyond.
-        One host read per version of the frozen read-out."""
+        """Exponent of the g_u image ('f16x2'): |g_u| <= sum_k |g_o| |Wo| / 4 <= max|Wo| / (4 B) whenever sum_k |g_o| <= 1/B per
+        row: the mean-reduced SmoothL1 / Huber / L1 / BCE-with-logits / soft-margin / hinge losses (|g_o| <= 1/(B K)) and
+        KL divergence against targets in [0, 1].  2^4 of slack covers cross-entropy (sum_k |g_o| <= 2/B for probability
+        targets), MSE residuals above 1 and external losses; MSE and Poisson NLL are unbounded, and the store saturates
+        beyond the slack.  One host read per version of the frozen read-out."""
         w = self.i2o.weight
         key = (w.data_ptr(), w._version, batch)
         if getattr(self, '_gexp', None) is None or self._gexp[0] != key:
@@ -824,14 +826,46 @@ class DenseDCLLlayer(nn.Module):
 # ------------------------------------------------------------------------------------------------
 # optimiser / loss adapters
 # ------------------------------------------------------------------------------------------------
+NATIVE_LOSSES = ('SmoothL1Loss', 'HuberLoss', 'MSELoss', 'L1Loss', 'CrossEntropyLoss', 'BCEWithLogitsLoss',
+                 'MultiLabelSoftMarginLoss', 'SoftMarginLoss', 'KLDivLoss', 'PoissonNLLLoss', 'HingeEmbeddingLoss')
+
+
 def _loss_kind(crit):
-    if type(crit) is nn.SmoothL1Loss and getattr(crit, 'beta', 1.0) == 1.0 and crit.reduction == 'mean':
+    """The device loss kind of a criterion: instances of exactly these torch.nn classes with their default arguments
+    (NATIVE_LOSSES; mean reduction).  Anything else -- a subclass, other arguments -- is LOSS_EXTERNAL: the per-step API
+    takes its gradient from autograd, the window drivers refuse it."""
+    t = type(crit)
+    if getattr(crit, 'reduction', None) != 'mean':
+        return _lib.LOSS_EXTERNAL
+    if (t is nn.SmoothL1Loss and getattr(crit, 'beta', 1.0) == 1.0) or (t is nn.HuberLoss and crit.delta == 1.0):
         return _lib.LOSS_SMOOTHL1
-    if type(crit) is nn.MSELoss and crit.reduction == 'mean':
+    if t is nn.MSELoss:
         return _lib.LOSS_MSE
-    if type(crit) is nn.L1Loss and crit.reduction == 'mean':
+    if t is nn.L1Loss:
         return _lib.LOSS_L1
+    if t is nn.CrossEntropyLoss and crit.weight is None and crit.label_smoothing == 0.0 and crit.ignore_index == -100:
+        return _lib.LOSS_CROSS_ENTROPY
+    if (t is nn.BCEWithLogitsLoss and crit.weight is None and crit.pos_weight is None) or \
+            (t is nn.MultiLabelSoftMarginLoss and crit.weight is None):
+        return _lib.LOSS_BCE_LOGITS
+    if t is nn.SoftMarginLoss:
+        return _lib.LOSS_SOFT_MARGIN
+    if t is nn.KLDivLoss and not crit.log_target:
+        return _lib.LOSS_KL_DIV
+    if t is nn.PoissonNLLLoss and crit.log_input and not crit.full:
+        return _lib.LOSS_POISSON_NLL
+    if t is nn.HingeEmbeddingLoss and crit.margin == 1.0:
+        return _lib.LOSS_HINGE
     return _lib.LOSS_EXTERNAL
+
+
+def _step_loss_kind(crit, target, pred):
+    """_loss_kind for one per-step backward: the kinds added after the first three read the target as a [B,K] array like
+    the read-out, so any other target form (class indices for CrossEntropyLoss, a broadcast) goes through autograd."""
+    kind = _loss_kind(crit)
+    if kind > _lib.LOSS_EXTERNAL and tuple(target.shape) != tuple(pred.shape):
+        return _lib.LOSS_EXTERNAL
+    return kind
 
 
 def _is_plain_adam(opt):
@@ -940,10 +974,10 @@ class DCLLBase(nn.Module):
         args = _lib.TrainArgs()
         args.target = _lib.ptr(targ)
         keep = [targ]
-        kind = _loss_kind(self.crit)
+        kind = _step_loss_kind(self.crit, targ, outs['pvoutput'])
         args.loss_kind = kind
         if kind == _lib.LOSS_EXTERNAL:
-            # any other torch loss class: its gradient w.r.t. the [B,K] read-outs comes from autograd
+            # any other loss: its gradient w.r.t. the [B,K] read-outs comes from autograd
             pvo = outs['pvoutput'].detach().clone().requires_grad_(True)
             loss = self.crit(pvo, targ)
             if lay.output_layer:
@@ -995,7 +1029,7 @@ class DCLLBase(nn.Module):
         targ = _as_cuda_f32(target)
         dev = targ.device
         args = _lib.TrainArgs()
-        kind = _loss_kind(self.crit)
+        kind = _step_loss_kind(self.crit, targ, outs['pvoutput'])
         args.loss_kind = kind
         keep = [targ]
         if kind == _lib.LOSS_EXTERNAL:

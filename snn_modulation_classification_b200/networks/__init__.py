@@ -13,8 +13,8 @@ import torch
 import yaml
 
 from .. import _lib
-from ..dcll.pytorch_libdcll import (Conv2dDCLLlayer, DCLLClassification, SpikeCells, _as_cuda_f32, _fill_adam,
-                                    _is_plain_adam, _loss_kind, _store_steps, device)
+from ..dcll.pytorch_libdcll import (NATIVE_LOSSES, Conv2dDCLLlayer, DCLLClassification, SpikeCells, _as_cuda_f32,
+                                    _fill_adam, _is_plain_adam, _loss_kind, _store_steps, device)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -189,7 +189,8 @@ class ConvNetwork(torch.nn.Module):
                     raise NotImplementedError('learn_window needs torch.optim.Adam slices; use learn() per timestep')
                 kind = _loss_kind(s.crit)
                 if kind == _lib.LOSS_EXTERNAL:
-                    raise NotImplementedError('learn_window implements SmoothL1Loss / MSELoss / L1Loss; use learn()')
+                    raise NotImplementedError('learn_window implements %s with default arguments; use learn()'
+                                              % ', '.join(NATIVE_LOSSES))
                 trains[i].loss_kind, trains[i].apply_update = kind, 1
                 st = [_fill_adam(trains[i].adam_i2h, s.optimizer, lay.i2h.weight, lay.i2h.bias)]
                 if lay.output_layer:
@@ -288,7 +289,7 @@ class ConvNetwork(torch.nn.Module):
             if not (_is_plain_adam(s.optimizer) and (not lay.output_layer or _is_plain_adam(s.optimizer2))):
                 raise NotImplementedError('learn_window_dp needs torch.optim.Adam slices')
             if _loss_kind(s.crit) == _lib.LOSS_EXTERNAL:
-                raise NotImplementedError('learn_window_dp implements SmoothL1Loss / MSELoss / L1Loss')
+                raise NotImplementedError('learn_window_dp implements %s with default arguments' % ', '.join(NATIVE_LOSSES))
         win = self._window_buffers(batch)
         Layers, Trains = _lib.ConvLayer * n, _lib.TrainArgs * n
         layers, trains = Layers(), Trains()
