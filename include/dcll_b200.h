@@ -60,6 +60,22 @@ typedef struct dcll_adam {
     float *m_b, *v_b;      /* device: exp_avg / exp_avg_sq of the bias   */
 } dcll_adam;
 
+/* Update rule of one dcll_adam, for the _opt entry points (train.py --optim_type): the dcll_adam keeps lr, betas, eps,
+ * weight_decay, step and the two float32 state tensors per parameter (exp_avg, and exp_avg_sq -- or exp_inf for Adamax,
+ * in v_w / v_b).  Each rule follows torch's _single_tensor_<rule> operation order.
+ *   ADAM   torch.optim.Adam (the entry points without _opt)
+ *   ADAMW  torch.optim.AdamW, or Adam(decoupled_weight_decay=True); amsgrad=False
+ *   ADAMAX torch.optim.Adamax
+ *   NADAM  torch.optim.NAdam (decoupled_wd, momentum_decay; mu_product in/out)
+ *   RADAM  torch.optim.RAdam (decoupled_wd)                                                                             */
+enum { DCLL_OPT_ADAM = 0, DCLL_OPT_ADAMW = 1, DCLL_OPT_ADAMAX = 2, DCLL_OPT_NADAM = 3, DCLL_OPT_RADAM = 4 };
+typedef struct dcll_optim {
+    int32_t kind;          /* DCLL_OPT_*                                                                    */
+    int32_t decoupled_wd;  /* NAdam / RAdam: decoupled_weight_decay (AdamW: always decoupled)              */
+    double momentum_decay; /* NAdam                                                                         */
+    float mu_product;      /* NAdam: torch's float32 state['mu_product'], before the call / after it        */
+} dcll_optim;
+
 /* One Conv2dDCLLlayer (dcll/pytorch_libdcll.py:512-612) with its i2h core
  * (ContinuousConv2D :296-429 or ContinuousRelativeRefractoryConv2D :432-509). */
 typedef struct dcll_conv_layer {
@@ -194,6 +210,10 @@ int dcll_conv_core_fwd(dcll_conv_layer *L, const void *x, void *stream);
 int dcll_conv_step_bwd_update(dcll_conv_layer *L, dcll_train_args *a, void *stream);
 /* Adam on gradients already in a->grad_* (data-parallel path, after the allreduce) */
 int dcll_conv_apply_update(dcll_conv_layer *L, dcll_train_args *a, void *stream);
+/* The same two calls with the update rules opt[0] (adam_i2h) and opt[1] (adam_out).  opt == NULL, or kind DCLL_OPT_ADAM,
+ * is Adam exactly as above.  Writes back step (in dcll_adam) and mu_product (in opt) of every rule it applied. */
+int dcll_conv_step_bwd_update_opt(dcll_conv_layer *L, dcll_train_args *a, dcll_optim *opt, void *stream);
+int dcll_conv_apply_update_opt(dcll_conv_layer *L, dcll_train_args *a, dcll_optim *opt, void *stream);
 
 /* -- dense layer: DenseDCLLlayer (dcll/pytorch_libdcll.py:198-266) over CLLDenseModule (:72-148) or
  *    CLLDenseRRPModule (:151-195).  Not instantiated by any entry point of the reference; FP32 tiled GEMMs. */
@@ -217,6 +237,8 @@ int dcll_dense_step_fwd(dcll_dense_layer *L, const float *x, int32_t *clout, voi
 /* local gradient (SURVEY appendix C: gW = ((g_o Wo) * s(1-s))^T eps1) + Adam on weight/bias when apply_update;
  * gradients are always left in grad_w / grad_b. */
 int dcll_dense_step_bwd_update(dcll_dense_layer *L, dcll_train_args *a, void *stream);
+/* the same with the update rule opt[0] of adam_i2h (NULL: Adam) */
+int dcll_dense_step_bwd_update_opt(dcll_dense_layer *L, dcll_train_args *a, dcll_optim *opt, void *stream);
 
 /* -- whole window: the T-loop of train.py:249-251 / test_radio_ml.py:144-145 ----------------- *
  * Runs `T` timesteps of ConvNetwork.learn (train != 0) or .test over `n_layers` chained
@@ -234,6 +256,11 @@ int dcll_net_window(dcll_conv_layer *layers, dcll_train_args *train, int n_layer
 int dcll_net_window_stats(dcll_conv_layer *layers, dcll_train_args *train, int n_layers, const void *x0,
                           const float *target, int64_t target_t_stride, int T, int train_mode, int burnin,
                           const int32_t *iter0, int32_t *clout, int32_t *hist, int hist_every, int hist_cap, void *stream);
+/* the same with update rules opt[2*l] (train[l].adam_i2h) and opt[2*l+1] (train[l].adam_out); NULL: Adam everywhere.  A NAdam
+ * mu_product is carried across the timesteps of the window and written back at the end. */
+int dcll_net_window_stats_opt(dcll_conv_layer *layers, dcll_train_args *train, dcll_optim *opt, int n_layers, const void *x0,
+                              const float *target, int64_t target_t_stride, int T, int train_mode, int burnin,
+                              const int32_t *iter0, int32_t *clout, int32_t *hist, int hist_every, int hist_cap, void *stream);
 
 /* -- data-parallel window (SURVEY.md section 8e; the reference has no multi-GPU code: train.py:249-251 over a batch shard) -- *
  * One process per GPU, identical weights, each rank its own B/world samples.  dcll_net_window_dp is dcll_net_window in
@@ -251,6 +278,10 @@ int dcll_dp_destroy(dcll_dp *dp);
 int dcll_net_window_dp(dcll_dp *dp, dcll_conv_layer *layers, dcll_train_args *train, int n_layers, const void *x0,
                        const float *target, int64_t target_t_stride, int T, int burnin, const int32_t *iter0, int32_t *clout,
                        float *const *bucket, const size_t *bucket_floats, void *stream);
+/* the same with update rules opt[2*l], opt[2*l+1] as in dcll_net_window_stats_opt */
+int dcll_net_window_dp_opt(dcll_dp *dp, dcll_conv_layer *layers, dcll_train_args *train, dcll_optim *opt, int n_layers,
+                           const void *x0, const float *target, int64_t target_t_stride, int T, int burnin, const int32_t *iter0,
+                           int32_t *clout, float *const *bucket, const size_t *bucket_floats, void *stream);
 
 /* -- multi-timestep inference of the radio_ml_conv stack on a 16x16 plane (test_radio_ml.py:144-145, script geometry) -- *
  * One launch runs Tc timesteps of the three conv cores (1->32, 32->32, 32->32; 7x7, padding 3, no pooling) with one CTA

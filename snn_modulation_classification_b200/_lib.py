@@ -16,6 +16,7 @@ X_DENSE, X_CELLS = 0, 1
 LOSS_SMOOTHL1, LOSS_MSE, LOSS_L1, LOSS_EXTERNAL = 0, 1, 2, 3
 LOSS_CROSS_ENTROPY, LOSS_BCE_LOGITS, LOSS_SOFT_MARGIN, LOSS_KL_DIV, LOSS_POISSON_NLL, LOSS_HINGE = 4, 5, 6, 7, 8, 9
 PREC_FP32, PREC_BF16X3, PREC_F16X2 = 0, 1, 2
+OPT_ADAM, OPT_ADAMW, OPT_ADAMAX, OPT_NADAM, OPT_RADAM = 0, 1, 2, 3, 4
 
 _fp = C.c_void_p  # device pointers travel as integers
 
@@ -24,6 +25,10 @@ class Adam(C.Structure):
     _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
                 ("weight_decay", C.c_double), ("step", C.c_int64),
                 ("m_w", _fp), ("v_w", _fp), ("m_b", _fp), ("v_b", _fp)]
+
+
+class Optim(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("decoupled_wd", C.c_int32), ("momentum_decay", C.c_double), ("mu_product", C.c_float)]
 
 
 class ConvLayer(C.Structure):
@@ -102,6 +107,13 @@ def _load():
         "dcll_dp_destroy": [_fp],
         "dcll_net_window_dp": [_fp, P(ConvLayer), P(TrainArgs), C.c_int, _fp, _fp, C.c_int64, C.c_int, C.c_int, P(C.c_int32), _fp,
                                P(_fp), P(C.c_size_t), _fp],
+        "dcll_conv_step_bwd_update_opt": [P(ConvLayer), P(TrainArgs), P(Optim), _fp],
+        "dcll_conv_apply_update_opt": [P(ConvLayer), P(TrainArgs), P(Optim), _fp],
+        "dcll_dense_step_bwd_update_opt": [P(DenseLayer), P(TrainArgs), P(Optim), _fp],
+        "dcll_net_window_stats_opt": [P(ConvLayer), P(TrainArgs), P(Optim), C.c_int, _fp, _fp, C.c_int64, C.c_int, C.c_int,
+                                      C.c_int, P(C.c_int32), _fp, _fp, C.c_int, C.c_int, _fp],
+        "dcll_net_window_dp_opt": [_fp, P(ConvLayer), P(TrainArgs), P(Optim), C.c_int, _fp, _fp, C.c_int64, C.c_int, C.c_int,
+                                   P(C.c_int32), _fp, P(_fp), P(C.c_size_t), _fp],
         "dcll_quantize": [_fp, C.c_int, C.c_int, _fp, _fp, _fp],
         "dcll_dequantize": [_fp, _fp, C.c_int, C.c_int, _fp, _fp],
     }
@@ -144,7 +156,9 @@ EXPORTS = ["dcll_launch_count", "dcll_profile_enable", "dcll_profile_read", "dcl
            "dcll_conv_core_fwd", "dcll_conv_step_bwd_update", "dcll_conv_apply_update", "dcll_net_window", "dcll_vote",
            "dcll_quantize", "dcll_dequantize", "dcll_sizeof_dense_layer", "dcll_dense_step_fwd",
            "dcll_dense_step_bwd_update", "dcll_net_window_stats", "dcll_infer_stack16", "dcll_conv_readout_rows", "dcll_conv_step_fwd_chain",
-           "dcll_conv_chain_fusable", "dcll_dp_unique_id", "dcll_dp_create", "dcll_dp_destroy", "dcll_net_window_dp", "dcll_image_encode", "dcll_debug_timeline"]
+           "dcll_conv_chain_fusable", "dcll_dp_unique_id", "dcll_dp_create", "dcll_dp_destroy", "dcll_net_window_dp", "dcll_image_encode", "dcll_debug_timeline",
+           "dcll_conv_step_bwd_update_opt", "dcll_conv_apply_update_opt", "dcll_dense_step_bwd_update_opt",
+           "dcll_net_window_stats_opt", "dcll_net_window_dp_opt"]
 
 
 def check(rc):

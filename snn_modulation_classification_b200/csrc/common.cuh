@@ -223,10 +223,12 @@ bool readout_tc_supported(const dcll_conv_layer *L);
 int readout_tc_blocks(const dcll_conv_layer *L);
 int launch_readout_tc(const dcll_conv_layer *L, float *partial, cudaStream_t st);   // tcgen05, split-bf16 x3
 int launch_loss_grad(const dcll_conv_layer *L, const float *target, int loss_kind, float *loss_out, cudaStream_t st);
-int launch_readout_bwd(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st);
+// so_out / so_i2h: the rule of adam_out / adam_i2h when it is not Adam (null: the Adam kernels)
+struct OptScalars;
+int launch_readout_bwd(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st, const OptScalars *so_out = nullptr);
 bool readout_bwd_tc_supported(const dcll_conv_layer *L, int hw, int F);                   // readout_bwd_tc.cu (DCLL_RB_TC=1)
 int launch_readout_bwd_tc(const dcll_conv_layer *L, const float *g_o, int hw, int F, float g_scale, cudaStream_t st);
-int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st);
+int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st, const OptScalars *so_i2h = nullptr);
 int wgrad_splits(const dcll_conv_layer *L);
 bool wgrad_tc_supported(const dcll_conv_layer *L);
 int wgrad_tc_splits(const dcll_conv_layer *L);
@@ -256,6 +258,62 @@ __device__ __forceinline__ void adam_elem(float &w, float g, float &m, float &v,
     float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), s.bc2_sqrt), s.eps);
     w = __fadd_rn(w, __fdiv_rn(__fmul_rn(s.neg_step_size, m), denom)); // addcdiv_(m, denom, -step_size)
 }
+
+// Scalars of one step of an AdamW / Adamax / NAdam / RAdam rule (dcll_optim), computed on the host in double exactly as torch's
+// _single_tensor_<rule> (net.cu: opt_scalars).  Each float is the python float rounded as torch rounds it when it meets a
+// float32 tensor.  c0..c3 by kind:
+//   ADAMW   -step_size, sqrt(bc2)                   ADAMAX  -lr / bc1
+//   NADAM   bc2, addcdiv value of grad, of exp_avg  RADAM   bc1, lr, sqrt(bc2), rect
+struct OptScalars {
+    int kind;                  // DCLL_OPT_*, never DCLL_OPT_ADAM (that rule runs adam_elem)
+    int rect;                  // RAdam: rho_t > 5 (decided on the host, uniform across the launch)
+    float decay;               // decoupled weight decay: param.mul_(1 - lr * weight_decay); 1 = none
+    float wd;                  // coupled weight decay: grad.add(param, alpha=weight_decay); 0 = none
+    float one_minus_beta1, beta2, one_minus_beta2, eps;
+    float c0, c1, c2, c3;
+};
+// step_after: the step count after this update; *mu_product (NAdam) is torch's float32 state, updated in place
+OptScalars opt_scalars(const dcll_adam &a, const dcll_optim &o, int64_t step_after, float *mu_product);
+// the scalars of slot o's next update (step a.step + 1) in *buf, or null when the slot runs Adam; advances o->mu_product
+const OptScalars *next_opt_scalars(const dcll_adam &a, dcll_optim *o, OptScalars *buf);
+
+__device__ __forceinline__ void opt_elem(float &w, float g, float &m, float &v, const OptScalars &s) {
+    if (s.decay != 1.f) w = __fmul_rn(w, s.decay);                   // param.mul_(1 - lr * weight_decay)
+    if (s.wd != 0.f) g = __fmaf_rn(s.wd, w, g);                       // grad.add(param, alpha=wd)
+    // exp_avg.lerp_(grad, 1-beta1), as adam_elem
+    if (s.one_minus_beta1 < 0.5f) m = __fmaf_rn(s.one_minus_beta1, __fsub_rn(g, m), m);
+    else m = __fsub_rn(g, __fmul_rn(__fsub_rn(g, m), __fsub_rn(1.f, s.one_minus_beta1)));
+    if (s.kind == DCLL_OPT_ADAMAX) {
+        v = fmaxf(__fmul_rn(v, s.beta2), __fadd_rn(fabsf(g), s.eps));  // maximum(exp_inf.mul_(beta2), grad.abs().add_(eps))
+        w = __fadd_rn(w, __fdiv_rn(__fmul_rn(s.c0, m), v));            // addcdiv_(exp_avg, exp_inf, value=-clr)
+        return;
+    }
+    // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value=1-beta2)
+    v = __fadd_rn(__fmul_rn(v, s.beta2), __fmul_rn(__fmul_rn(s.one_minus_beta2, g), g));
+    if (s.kind == DCLL_OPT_NADAM) {
+        const float denom = __fadd_rn(__fsqrt_rn(__fdiv_rn(v, s.c0)), s.eps);   // exp_avg_sq.div(bc2).sqrt().add_(eps)
+        w = __fadd_rn(w, __fdiv_rn(__fmul_rn(s.c1, g), denom));                 // addcdiv_(grad, denom, -lr(1-mu)/(1-mu_product))
+        w = __fadd_rn(w, __fdiv_rn(__fmul_rn(s.c2, m), denom));                 // addcdiv_(exp_avg, denom, -lr mu_next/(1-mu_product_next))
+    } else if (s.kind == DCLL_OPT_RADAM) {
+        float u = __fmul_rn(__fdiv_rn(m, s.c0), s.c1);                          // exp_avg / bc1 * lr
+        // * (sqrt(bc2) / (sqrt(v) + eps)) * rect; a python float over a tensor is reciprocal() * float in torch
+        if (s.rect) u = __fmul_rn(__fmul_rn(u, __fmul_rn(__frcp_rn(__fadd_rn(__fsqrt_rn(v), s.eps)), s.c2)), s.c3);
+        w = __fsub_rn(w, u);                                                    // param.add_(update, alpha=-1)
+    } else {                                                                    // DCLL_OPT_ADAMW: Adam after the decay
+        const float denom = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), s.c1), s.eps);
+        w = __fadd_rn(w, __fdiv_rn(__fmul_rn(s.c0, m), denom));
+    }
+}
+
+// the element update of a kernel body shared by the Adam kernel and its _opt sibling
+__device__ __forceinline__ void elem_update(float &w, float g, float &m, float &v, const AdamScalars &s) { adam_elem(w, g, m, v, s); }
+__device__ __forceinline__ void elem_update(float &w, float g, float &m, float &v, const OptScalars &s) { opt_elem(w, g, m, v, s); }
+// the rule of an optimizer slot: null or DCLL_OPT_ADAM is Adam (the pre-existing kernels)
+static inline bool opt_active(const dcll_optim *o) { return o && o->kind != DCLL_OPT_ADAM; }
+int launch_opt_flat(float *w, const float *g, float *m, float *v, size_t n, const OptScalars &sc, cudaStream_t st);
+// Adam or the rule o over two flat parameters (weight, bias), then step += 1 (net.cu; the dense layer's update)
+int dense_flat_update(dcll_adam &a, dcll_optim *o, float *w, const float *gw, size_t nw, float *b, const float *gb, size_t nb,
+                      cudaStream_t st);
 
 __device__ __forceinline__ float sigmoidf_ref(float x) {
     // 1/(1+exp(-x)) with IEEE division: matches torch-CPU sigmoid to ~1 ulp

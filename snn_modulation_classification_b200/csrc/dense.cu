@@ -181,8 +181,16 @@ extern "C" __attribute__((visibility("default"))) int dcll_dense_step_fwd(dcll_d
 
 extern "C" __attribute__((visibility("default"))) int dcll_dense_step_bwd_update(dcll_dense_layer *L, dcll_train_args *a,
                                                                                   void *stream) {
+    return dcll_dense_step_bwd_update_opt(L, a, nullptr, stream);
+}
+
+// opt: the update rule of adam_i2h, or null (Adam)
+extern "C" __attribute__((visibility("default"))) int dcll_dense_step_bwd_update_opt(dcll_dense_layer *L, dcll_train_args *a,
+                                                                                      dcll_optim *opt, void *stream) {
     int rc = check_dense(L, "dcll_dense_step_bwd_update");
     if (rc != DCLL_OK) return rc;
+    DCLL_REQUIRE(!opt || (opt->kind >= DCLL_OPT_ADAM && opt->kind <= DCLL_OPT_RADAM), DCLL_EINVAL,
+                 "dcll_dense_step_bwd_update_opt: unknown update rule");
     DCLL_REQUIRE(a && L->g_o && L->g_u && L->grad_w && L->grad_b, DCLL_EINVAL, "dcll_dense_step_bwd_update: null scratch");
     cudaStream_t st = (cudaStream_t)stream;
     const int nk = L->B * L->K;
@@ -213,12 +221,8 @@ extern "C" __attribute__((visibility("default"))) int dcll_dense_step_bwd_update
     if (a->apply_update) {
         DCLL_REQUIRE(a->adam_i2h.m_w && a->adam_i2h.v_w && a->adam_i2h.m_b && a->adam_i2h.v_b, DCLL_EINVAL,
                      "dcll_dense_step_bwd_update: null Adam state");
-        AdamScalars sc = adam_scalars(a->adam_i2h, a->adam_i2h.step + 1);
-        rc = launch_adam_flat(L->weight, L->grad_w, a->adam_i2h.m_w, a->adam_i2h.v_w, (size_t)L->Out * L->In, sc, st);
+        rc = dense_flat_update(a->adam_i2h, opt, L->weight, L->grad_w, (size_t)L->Out * L->In, L->bias, L->grad_b, (size_t)L->Out, st);
         if (rc != DCLL_OK) return rc;
-        rc = launch_adam_flat(L->bias, L->grad_b, a->adam_i2h.m_b, a->adam_i2h.v_b, (size_t)L->Out, sc, st);
-        if (rc != DCLL_OK) return rc;
-        a->adam_i2h.step += 1;
     }
     return DCLL_OK;
 }

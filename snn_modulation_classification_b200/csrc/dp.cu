@@ -25,10 +25,11 @@
 namespace dcll {
 
 // defined in wgrad.cu / net.cu
-int launch_bucket_adam(const dcll_conv_layer *L, dcll_train_args *a, const float *bucket, cudaStream_t st);
+int launch_bucket_adam(const dcll_conv_layer *L, dcll_train_args *a, const float *bucket, cudaStream_t st, dcll_optim *opt);
 int dp_step_fwd(dcll_conv_layer *L, const void *x, const float *target, int loss_kind, int32_t *clout, cudaStream_t st,
                 const dcll_conv_layer *next, bool trace_done, int spike_io, int layer);
 int dp_step_bwd(dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st, int layer);
+int dp_check_opt(const dcll_optim *opt, int n_layers);
 int dp_check(const dcll_conv_layer *layers, const dcll_train_args *train, int n_layers);
 
 struct NcclApi {
@@ -138,10 +139,23 @@ extern "C" __attribute__((visibility("default"))) int dcll_net_window_dp(dcll_dp
                                                                           const void *x0, const float *target, int64_t target_t_stride, int T,
                                                                           int burnin, const int32_t *iter0, int32_t *clout,
                                                                           float *const *bucket, const size_t *bucket_floats, void *stream) {
+    return dcll_net_window_dp_opt(dp, layers, train, nullptr, n_layers, x0, target, target_t_stride, T, burnin, iter0, clout, bucket,
+                                  bucket_floats, stream);
+}
+
+// opt: the update rules opt[2l] (train[l].adam_i2h) and opt[2l + 1] (train[l].adam_out), or null (Adam everywhere)
+extern "C" __attribute__((visibility("default"))) int dcll_net_window_dp_opt(dcll_dp *dp, dcll_conv_layer *layers, dcll_train_args *train,
+                                                                              dcll_optim *opt, int n_layers, const void *x0,
+                                                                              const float *target, int64_t target_t_stride, int T,
+                                                                              int burnin, const int32_t *iter0, int32_t *clout,
+                                                                              float *const *bucket, const size_t *bucket_floats,
+                                                                              void *stream) {
     DCLL_REQUIRE(dp && dp->comm && layers && train && n_layers > 0 && n_layers <= 16 && x0 && target && T > 0 && iter0 && bucket && bucket_floats,
                  DCLL_EINVAL, "dcll_net_window_dp: bad arguments");
     set_reserved_sms(0);
     int rc = dp_check(layers, train, n_layers);
+    if (rc != DCLL_OK) return rc;
+    rc = dp_check_opt(opt, n_layers);
     if (rc != DCLL_OK) return rc;
     for (int l = 0; l < n_layers; ++l) {
         const dcll_conv_layer &L = layers[l];
@@ -168,7 +182,7 @@ extern "C" __attribute__((visibility("default"))) int dcll_net_window_dp(dcll_dp
         DCLL_CUDA_OK(cudaStreamWaitEvent(st, dp->ev_red[l], 0));
         pending[l] = false;
         reserve();
-        return launch_bucket_adam(&layers[l], &train[l], bucket[l], st);
+        return launch_bucket_adam(&layers[l], &train[l], bucket[l], st, opt ? opt + 2 * l : nullptr);
     };
     for (int t = 0; t < T; ++t) {
         const float *tgt = target + (size_t)t * target_t_stride;

@@ -101,6 +101,60 @@ AdamScalars adam_scalars(const dcll_adam &a, int64_t step_after) {
     return s;
 }
 
+OptScalars opt_scalars(const dcll_adam &a, const dcll_optim &o, int64_t step_after, float *mu_product) {
+    // torch/optim/{adam,adamax,nadam,radam}.py (_single_tensor_*), python-float arithmetic on the float32 step count
+    const double t = (double)step_after, lr = a.lr, b1 = a.beta1, b2 = a.beta2, wd = a.weight_decay;
+    const bool decoupled = o.kind == DCLL_OPT_ADAMW || ((o.kind == DCLL_OPT_NADAM || o.kind == DCLL_OPT_RADAM) && o.decoupled_wd);
+    OptScalars s = {};
+    s.kind = o.kind;
+    s.decay = (decoupled && wd != 0.0) ? (float)(1.0 - lr * wd) : 1.f;
+    s.wd = decoupled ? 0.f : (float)wd;
+    s.one_minus_beta1 = (float)(1.0 - b1);
+    s.beta2 = (float)b2;
+    s.one_minus_beta2 = (float)(1.0 - b2);
+    s.eps = (float)a.eps;
+    const double bc1 = 1.0 - pow(b1, t), bc2 = 1.0 - pow(b2, t);
+    if (o.kind == DCLL_OPT_ADAMW) {
+        s.c0 = (float)(-(lr / bc1));
+        s.c1 = (float)sqrt(bc2);
+    } else if (o.kind == DCLL_OPT_ADAMAX) {
+        s.c0 = (float)(-(lr / bc1));
+    } else if (o.kind == DCLL_OPT_NADAM) {
+        const double mu = b1 * (1.0 - 0.5 * pow(0.96, t * o.momentum_decay));
+        const double mu_next = b1 * (1.0 - 0.5 * pow(0.96, (t + 1.0) * o.momentum_decay));
+        *mu_product = *mu_product * (float)mu;                    // mu_product *= mu: a float32 tensor times a python float
+        const double mp = (double)*mu_product, mp_next = mp * mu_next;
+        s.c0 = (float)bc2;
+        s.c1 = (float)(-lr * (1.0 - mu) / (1.0 - mp));
+        s.c2 = (float)((-lr * mu_next) / (1.0 - mp_next));
+    } else {                                                        // DCLL_OPT_RADAM
+        const double rho_inf = 2.0 / (1.0 - b2) - 1.0;
+        const double rho_t = rho_inf - 2.0 * t * pow(b2, t) / bc2;
+        s.rect = rho_t > 5.0;
+        s.c0 = (float)bc1;
+        s.c1 = (float)lr;
+        if (s.rect) {
+            s.c2 = (float)pow(bc2, 0.5);
+            s.c3 = (float)pow((rho_t - 4.0) * (rho_t - 2.0) * rho_inf / ((rho_inf - 4.0) * (rho_inf - 2.0) * rho_t), 0.5);
+        }
+    }
+    return s;
+}
+
+const OptScalars *next_opt_scalars(const dcll_adam &a, dcll_optim *o, OptScalars *buf) {
+    if (!opt_active(o)) return nullptr;
+    *buf = opt_scalars(a, *o, a.step + 1, &o->mu_product);
+    return buf;
+}
+
+static int check_opt(const dcll_optim *opt, int n, const char *who) {
+    for (int i = 0; opt && i < n; ++i)
+        DCLL_REQUIRE(opt[i].kind >= DCLL_OPT_ADAM && opt[i].kind <= DCLL_OPT_RADAM, DCLL_EINVAL, "%s: unknown update rule %d", who,
+                     opt[i].kind);
+    return DCLL_OK;
+}
+int dp_check_opt(const dcll_optim *opt, int n_layers) { return check_opt(opt, 2 * n_layers, "dcll_net_window_dp_opt"); }
+
 static int check_layer(const dcll_conv_layer *L, const char *who) {
     DCLL_REQUIRE(L, DCLL_EINVAL, "%s: null layer", who);
     DCLL_REQUIRE(L->B > 0 && L->Cin > 0 && L->H > 0 && L->W > 0 && L->Cout > 0 && L->K > 0, DCLL_EINVAL,
@@ -170,16 +224,23 @@ static int step_fwd(dcll_conv_layer *L, const void *x, const float *target, int 
     return launch_readout_fwd(L, target, loss_kind, clout, loss_out, st);
 }
 
-static int step_bwd(dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st) {
+// opt: the rules of adam_i2h / adam_out, or null (Adam)
+static int step_bwd(dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st, dcll_optim *opt = nullptr) {
     int rc;
+    OptScalars buf_i2h, buf_out;
+    const OptScalars *so_i2h = nullptr, *so_out = nullptr;
+    if (a->apply_update && opt) {
+        so_i2h = next_opt_scalars(a->adam_i2h, &opt[0], &buf_i2h);
+        if (L->output_layer) so_out = next_opt_scalars(a->adam_out, &opt[1], &buf_out);
+    }
     {
         ProfScope ps(KC_READOUT_BWD, g_layer, st);
-        rc = launch_readout_bwd(L, a, st);
+        rc = launch_readout_bwd(L, a, st, so_out);
     }
     if (rc != DCLL_OK) return rc;
     {
         ProfScope ps(KC_WGRAD, g_layer, st);
-        rc = launch_wgrad(L, a, st);
+        rc = launch_wgrad(L, a, st, so_i2h);
     }
     if (rc != DCLL_OK) return rc;
     if (a->apply_update) {
@@ -386,9 +447,16 @@ extern "C" __attribute__((visibility("default"))) int dcll_conv_core_fwd(dcll_co
 }
 
 extern "C" __attribute__((visibility("default"))) int dcll_conv_step_bwd_update(dcll_conv_layer *L, dcll_train_args *a, void *stream) {
+    return dcll_conv_step_bwd_update_opt(L, a, nullptr, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int dcll_conv_step_bwd_update_opt(dcll_conv_layer *L, dcll_train_args *a, dcll_optim *opt,
+                                                                                     void *stream) {
     int rc = check_layer(L, "dcll_conv_step_bwd_update");
     if (rc != DCLL_OK) return rc;
     rc = check_train(L, a, "dcll_conv_step_bwd_update");
+    if (rc != DCLL_OK) return rc;
+    rc = check_opt(opt, 2, "dcll_conv_step_bwd_update_opt");
     if (rc != DCLL_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (a->loss_kind == DCLL_LOSS_EXTERNAL) {
@@ -403,31 +471,50 @@ extern "C" __attribute__((visibility("default"))) int dcll_conv_step_bwd_update(
         rc = launch_loss_grad(L, a->target, a->loss_kind, a->loss_out, st);
         if (rc != DCLL_OK) return rc;
     }
-    return step_bwd(L, a, st);
+    return step_bwd(L, a, st, opt);
+}
+
+// Adam, or the rule of the slot, over flat parameters (w, b) with gradients (gw, gb)
+static int flat_update(dcll_adam &a, dcll_optim *o, float *w, const float *gw, size_t nw, float *b, const float *gb, size_t nb,
+                       cudaStream_t st) {
+    OptScalars buf;
+    const OptScalars *so = next_opt_scalars(a, o, &buf);
+    const AdamScalars sc = adam_scalars(a, a.step + 1);
+    int rc = so ? launch_opt_flat(w, gw, a.m_w, a.v_w, nw, *so, st) : launch_adam_flat(w, gw, a.m_w, a.v_w, nw, sc, st);
+    if (rc != DCLL_OK) return rc;
+    rc = so ? launch_opt_flat(b, gb, a.m_b, a.v_b, nb, *so, st) : launch_adam_flat(b, gb, a.m_b, a.v_b, nb, sc, st);
+    if (rc != DCLL_OK) return rc;
+    a.step += 1;
+    return DCLL_OK;
 }
 
 extern "C" __attribute__((visibility("default"))) int dcll_conv_apply_update(dcll_conv_layer *L, dcll_train_args *a, void *stream) {
+    return dcll_conv_apply_update_opt(L, a, nullptr, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int dcll_conv_apply_update_opt(dcll_conv_layer *L, dcll_train_args *a, dcll_optim *opt,
+                                                                                  void *stream) {
     int rc = check_layer(L, "dcll_conv_apply_update");
     if (rc != DCLL_OK) return rc;
     DCLL_REQUIRE(a && a->grad_w && a->grad_b, DCLL_EINVAL, "dcll_conv_apply_update: null gradients");
+    rc = check_opt(opt, 2, "dcll_conv_apply_update_opt");
+    if (rc != DCLL_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     Geo g = geo_of(L);
-    AdamScalars sc = adam_scalars(a->adam_i2h, a->adam_i2h.step + 1);
-    rc = launch_adam_flat(L->weight, a->grad_w, a->adam_i2h.m_w, a->adam_i2h.v_w, (size_t)g.nW, sc, st);
+    rc = flat_update(a->adam_i2h, opt, L->weight, a->grad_w, (size_t)g.nW, L->bias, a->grad_b, (size_t)L->Cout, st);
     if (rc != DCLL_OK) return rc;
-    rc = launch_adam_flat(L->bias, a->grad_b, a->adam_i2h.m_b, a->adam_i2h.v_b, (size_t)L->Cout, sc, st);
-    if (rc != DCLL_OK) return rc;
-    a->adam_i2h.step += 1;
     if (L->output_layer) {
         DCLL_REQUIRE(a->grad_wout && a->grad_bout, DCLL_EINVAL, "dcll_conv_apply_update: null output_ gradients");
-        AdamScalars so = adam_scalars(a->adam_out, a->adam_out.step + 1);
-        rc = launch_adam_flat(L->wout, a->grad_wout, a->adam_out.m_w, a->adam_out.v_w, (size_t)L->K * g.F, so, st);
+        rc = flat_update(a->adam_out, opt ? opt + 1 : nullptr, L->wout, a->grad_wout, (size_t)L->K * g.F, L->bout, a->grad_bout,
+                         (size_t)L->K, st);
         if (rc != DCLL_OK) return rc;
-        rc = launch_adam_flat(L->bout, a->grad_bout, a->adam_out.m_b, a->adam_out.v_b, (size_t)L->K, so, st);
-        if (rc != DCLL_OK) return rc;
-        a->adam_out.step += 1;
     }
     return dcll_conv_sync_weights(L, stream);
+}
+
+int dcll::dense_flat_update(dcll_adam &a, dcll_optim *o, float *w, const float *gw, size_t nw, float *b, const float *gb, size_t nb,
+                      cudaStream_t st) {
+    return flat_update(a, o, w, gw, nw, b, gb, nb, st);
 }
 
 // 19 equal bins over [0,1], last bin closed on the right (numpy.histogram with bins = linspace(0,1,20)).
@@ -478,11 +565,22 @@ extern "C" __attribute__((visibility("default"))) int dcll_net_window(dcll_conv_
 extern "C" __attribute__((visibility("default"))) int dcll_net_window_stats(dcll_conv_layer *layers, dcll_train_args *train, int n_layers, const void *x0,
                                const float *target, int64_t target_t_stride, int T, int train_mode, int burnin,
                                const int32_t *iter0, int32_t *clout, int32_t *hist, int hist_every, int hist_cap, void *stream) {
+    return dcll_net_window_stats_opt(layers, train, nullptr, n_layers, x0, target, target_t_stride, T, train_mode, burnin, iter0, clout,
+                                     hist, hist_every, hist_cap, stream);
+}
+
+// opt: the update rules opt[2l] (train[l].adam_i2h) and opt[2l + 1] (train[l].adam_out), or null (Adam everywhere)
+extern "C" __attribute__((visibility("default"))) int dcll_net_window_stats_opt(dcll_conv_layer *layers, dcll_train_args *train, dcll_optim *opt,
+                               int n_layers, const void *x0, const float *target, int64_t target_t_stride, int T, int train_mode,
+                               int burnin, const int32_t *iter0, int32_t *clout, int32_t *hist, int hist_every, int hist_cap,
+                               void *stream) {
     DCLL_REQUIRE(layers && n_layers > 0 && x0 && T > 0 && iter0, DCLL_EINVAL, "dcll_net_window: bad arguments");
     DCLL_REQUIRE(!hist || (hist_every > 0 && hist_cap > 0), DCLL_EINVAL, "dcll_net_window: bad histogram arguments");
     int hist_n[16] = {0};
     DCLL_REQUIRE(!hist || n_layers <= 16, DCLL_EINVAL, "dcll_net_window: statistics support at most 16 layers");
     DCLL_REQUIRE(!train_mode || (train && target), DCLL_EINVAL, "dcll_net_window: training needs train args and a target");
+    int rc0 = check_opt(opt, 2 * n_layers, "dcll_net_window_stats_opt");
+    if (rc0 != DCLL_OK) return rc0;
     for (int l = 0; l < n_layers; ++l) {
         int rc = check_layer(&layers[l], "dcll_net_window");
         if (rc != DCLL_OK) return rc;
@@ -530,7 +628,7 @@ extern "C" __attribute__((visibility("default"))) int dcll_net_window_stats(dcll
                 DCLL_LAUNCH_OK("activity_hist_kernel");
             }
             if (do_train) {
-                rc = step_bwd(L, &train[l], st);
+                rc = step_bwd(L, &train[l], st, opt ? opt + 2 * l : nullptr);
                 if (rc != DCLL_OK) return rc;
             }
         }

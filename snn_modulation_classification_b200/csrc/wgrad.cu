@@ -188,11 +188,12 @@ __global__ void __launch_bounds__(8 * wg_ci_t(KH) * KH) wgrad_kernel(const WgP p
 //     next convolution must undo -- and slot 1 = the exponent for the next image from this step's maximum, and resets 2 and 3.
 //     It is the only writer of the slots, and by then every other block has read slot 1.
 constexpr int RED_U = 10;   // partial-block loads in flight per thread in the reducers below
+template <class Sc>
 __device__ __forceinline__ void reduce_adam_tail(float (&red)[4][64], int n_tot, int nW, int Cout, int CoutPad, int CinKK,
                                                  float *__restrict__ w, float *__restrict__ wt, float *__restrict__ bias,
                                                  float *__restrict__ m_w, float *__restrict__ v_w, float *__restrict__ m_b,
                                                  float *__restrict__ v_b, float *__restrict__ grad_w, float *__restrict__ grad_b, int apply,
-                                                 const AdamScalars &sc, __nv_bfloat16 *__restrict__ w_mma, int Cin, int KHKW, int KW,
+                                                 const Sc &sc, __nv_bfloat16 *__restrict__ w_mma, int Cin, int KHKW, int KW,
                                                  int *__restrict__ w_exp, int kexp, float w_pre, float m_pre, float v_pre) {
     const int e = threadIdx.x & 63, sl = threadIdx.x >> 6;
     const int i = blockIdx.x * 64 + e;
@@ -203,7 +204,7 @@ __device__ __forceinline__ void reduce_adam_tail(float (&red)[4][64], int n_tot,
             if (grad_w) grad_w[i] = g;
             if (apply) {
                 float wv = w_pre, m = m_pre, v = v_pre;                   // loaded by the caller BEFORE the reduction (one round trip less)
-                adam_elem(wv, g, m, v, sc);
+                elem_update(wv, g, m, v, sc);
                 w[i] = wv, m_w[i] = m, v_w[i] = v;
                 wabs = fabsf(wv);
                 int co = i / CinKK, r = i - co * CinKK;
@@ -231,7 +232,7 @@ __device__ __forceinline__ void reduce_adam_tail(float (&red)[4][64], int n_tot,
             if (grad_b) grad_b[co] = g;
             if (apply) {
                 float wv = bias[co], m = m_b[co], v = v_b[co];
-                adam_elem(wv, g, m, v, sc);
+                elem_update(wv, g, m, v, sc);
                 bias[co] = wv, m_b[co] = m, v_b[co] = v;
             }
         }
@@ -257,16 +258,17 @@ __device__ __forceinline__ void reduce_adam_tail(float (&red)[4][64], int n_tot,
     }
 }
 
+// parameters of the reducers' update tail (w, moments, gradients, kernel-side copies)
+#define RED_TAIL_PARAMS                                                                                                          \
+    float *__restrict__ w, float *__restrict__ wt, float *__restrict__ bias, float *__restrict__ m_w, float *__restrict__ v_w,   \
+        float *__restrict__ m_b, float *__restrict__ v_b, float *__restrict__ grad_w, float *__restrict__ grad_b, int apply
+#define RED_TAIL_PARAMS2 __nv_bfloat16 *__restrict__ w_mma, int Cin, int KHKW, int KW, int *__restrict__ w_exp
+#define RED_TAIL_ARGS w, wt, bias, m_w, v_w, m_b, v_b, grad_w, grad_b, apply, sc, w_mma, Cin, KHKW, KW, w_exp
+
 // grad = sum_s partial[s] (fixed order) ; Adam ; W, W^T, moments
-__global__ void __launch_bounds__(256) reduce_adam_kernel(const float *__restrict__ partial, int S, int n_tot, int nW,
-                                                          int Cout, int CoutPad, int CinKK, float *__restrict__ w,
-                                                          float *__restrict__ wt, float *__restrict__ bias,
-                                                          float *__restrict__ m_w, float *__restrict__ v_w,
-                                                          float *__restrict__ m_b, float *__restrict__ v_b,
-                                                          float *__restrict__ grad_w, float *__restrict__ grad_b, int apply,
-                                                          AdamScalars sc, __nv_bfloat16 *__restrict__ w_mma, int Cin, int KHKW, int KW,
-                                                          int *__restrict__ w_exp) {
-    pdl_entry();
+template <class Sc>
+__device__ __forceinline__ void reduce_body(const float *__restrict__ partial, int S, int n_tot, int nW, int Cout, int CoutPad,
+                                            int CinKK, RED_TAIL_PARAMS, const Sc &sc, RED_TAIL_PARAMS2) {
     // CTA = 64 elements x 4 slices of the partial blocks (a single serial walk over ~150 blocks was pure load latency);
     // the slices are combined in a fixed order, so the result stays bit-reproducible
     __shared__ float red[4][64];
@@ -295,21 +297,27 @@ __global__ void __launch_bounds__(256) reduce_adam_kernel(const float *__restric
     reduce_adam_tail(red, n_tot, nW, Cout, CoutPad, CinKK, w, wt, bias, m_w, v_w, m_b, v_b, grad_w, grad_b, apply, sc, w_mma, Cin, KHKW,
                      KW, w_exp, kexp, w_pre, m_pre, v_pre);
 }
+__global__ void __launch_bounds__(256) reduce_adam_kernel(const float *__restrict__ partial, int S, int n_tot, int nW, int Cout,
+                                                          int CoutPad, int CinKK, RED_TAIL_PARAMS, AdamScalars sc,
+                                                          RED_TAIL_PARAMS2) {
+    pdl_entry();
+    reduce_body(partial, S, n_tot, nW, Cout, CoutPad, CinKK, RED_TAIL_ARGS);
+}
+__global__ void __launch_bounds__(256) reduce_opt_kernel(const float *__restrict__ partial, int S, int n_tot, int nW, int Cout,
+                                                         int CoutPad, int CinKK, RED_TAIL_PARAMS, OptScalars sc, RED_TAIL_PARAMS2) {
+    pdl_entry();
+    reduce_body(partial, S, n_tot, nW, Cout, CoutPad, CinKK, RED_TAIL_ARGS);
+}
 
 // Same reduction + Adam tail for the partial blocks of wgrad_tc2_kernel (wgrad_tc2.cu): one compact block per CTA,
 //   block[(co*32 + ci)*20 + a*5 + slot],  a = kernel column within the role (A: kw 0..3, B: kw 4..6), slot <-> kh = 4g - 1 + slot,
 //   + 32 bias sums (role B blocks).  CTA c: pair c >> 1 (pairs [0, nA) = role A), kernel-row group g = c & 1.
 // Element (kh, kw) lives in the role's CTAs with g = 0 when kh <= 3 (slot kh + 1) and with g = 1 when kh >= 3 (slot kh - 3);
 // kh = 3 is the sum of both.  Blocks are walked in a fixed order by 4 slices that are combined in a fixed order.
-__global__ void __launch_bounds__(256) reduce_adam_rp_kernel(const float *__restrict__ partial, int nA, int nB, int blk, int nw_blk,
-                                                             int n_tot, int nW, int Cout, int CoutPad, int CinKK, float *__restrict__ w,
-                                                             float *__restrict__ wt, float *__restrict__ bias,
-                                                             float *__restrict__ m_w, float *__restrict__ v_w,
-                                                             float *__restrict__ m_b, float *__restrict__ v_b,
-                                                             float *__restrict__ grad_w, float *__restrict__ grad_b, int apply,
-                                                             AdamScalars sc, __nv_bfloat16 *__restrict__ w_mma, int Cin, int KHKW, int KW,
-                                                             int *__restrict__ w_exp) {
-    pdl_entry();
+template <class Sc>
+__device__ __forceinline__ void reduce_rp_body(const float *__restrict__ partial, int nA, int nB, int blk, int nw_blk, int n_tot,
+                                               int nW, int Cout, int CoutPad, int CinKK, RED_TAIL_PARAMS, const Sc &sc,
+                                               RED_TAIL_PARAMS2) {
     __shared__ float red[4][64];
     const int e = threadIdx.x & 63, sl = threadIdx.x >> 6;
     const int i = blockIdx.x * 64 + e;
@@ -358,6 +366,21 @@ __global__ void __launch_bounds__(256) reduce_adam_rp_kernel(const float *__rest
     reduce_adam_tail(red, n_tot, nW, Cout, CoutPad, CinKK, w, wt, bias, m_w, v_w, m_b, v_b, grad_w, grad_b, apply, sc, w_mma, Cin, KHKW,
                      KW, w_exp, kexp, w_pre, m_pre, v_pre);
 }
+__global__ void __launch_bounds__(256) reduce_adam_rp_kernel(const float *__restrict__ partial, int nA, int nB, int blk, int nw_blk,
+                                                             int n_tot, int nW, int Cout, int CoutPad, int CinKK, RED_TAIL_PARAMS,
+                                                             AdamScalars sc, RED_TAIL_PARAMS2) {
+    pdl_entry();
+    reduce_rp_body(partial, nA, nB, blk, nw_blk, n_tot, nW, Cout, CoutPad, CinKK, RED_TAIL_ARGS);
+}
+__global__ void __launch_bounds__(256) reduce_opt_rp_kernel(const float *__restrict__ partial, int nA, int nB, int blk, int nw_blk,
+                                                            int n_tot, int nW, int Cout, int CoutPad, int CinKK, RED_TAIL_PARAMS,
+                                                            OptScalars sc, RED_TAIL_PARAMS2) {
+    pdl_entry();
+    reduce_rp_body(partial, nA, nB, blk, nw_blk, n_tot, nW, Cout, CoutPad, CinKK, RED_TAIL_ARGS);
+}
+#undef RED_TAIL_PARAMS
+#undef RED_TAIL_PARAMS2
+#undef RED_TAIL_ARGS
 
 static int wg_n_ci_chunks(const dcll_conv_layer *L) {
     int ci_t = L->KH >= 7 ? 4 : (L->KH >= 5 ? 6 : (L->KH >= 3 ? 10 : 32));
@@ -409,19 +432,30 @@ static int launch_wg(const WgP &p, const dcll_conv_layer *L, cudaStream_t st) {
 
 // Adam on an already averaged gradient bucket [gW | gb | gWout | gbout] (data-parallel driver, dp.cu): the conv parameters go
 // through reduce_adam_kernel with the bucket as its single partial block, so weight_t and the tensor-core weight image are
-// refreshed by the same launch, as on the single-GPU path; output_ takes the flat kernel.
-int launch_bucket_adam(const dcll_conv_layer *L, dcll_train_args *a, const float *bucket, cudaStream_t st) {
+// refreshed by the same launch, as on the single-GPU path; output_ takes the flat kernel.  opt: the rules of adam_i2h, adam_out
+// (null: Adam).
+int launch_bucket_adam(const dcll_conv_layer *L, dcll_train_args *a, const float *bucket, cudaStream_t st, dcll_optim *opt) {
     Geo g = geo_of(L);
     const int n_tot = g.nW + L->Cout;
     {
+        OptScalars buf;
+        const OptScalars *so = next_opt_scalars(a->adam_i2h, opt, &buf);
         AdamScalars sc = adam_scalars(a->adam_i2h, a->adam_i2h.step + 1);
         dcll_adam &o = a->adam_i2h;
         ProfScope ps(KC_ADAM, 0, st);
-        launch_k(reduce_adam_kernel, ceil_div(n_tot, 64), 256, 0, st, bucket, 1, n_tot, g.nW, L->Cout, g.CoutPad, L->Cin * L->KH * L->KW,
-                 L->weight, L->weight_t, L->bias, o.m_w, o.v_w, o.m_b, o.v_b, (float *)nullptr, (float *)nullptr, 1, sc,
-                 L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma), L->Cin, L->KH * L->KW, L->KW,
-                 (prec_f16(L) && !L->quantized) ? L->w_exp : (int *)nullptr);   // F16X2: same image / exponent protocol as the single-GPU step
-        DCLL_LAUNCH_OK("reduce_adam_kernel");
+#define RED_BUCKET(KERN, SC)                                                                                                          \
+    launch_k(KERN, ceil_div(n_tot, 64), 256, 0, st, bucket, 1, n_tot, g.nW, L->Cout, g.CoutPad, L->Cin * L->KH * L->KW, L->weight,  \
+             L->weight_t, L->bias, o.m_w, o.v_w, o.m_b, o.v_b, (float *)nullptr, (float *)nullptr, 1, SC,                            \
+             L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma), L->Cin, L->KH * L->KW, L->KW,                \
+             (prec_f16(L) && !L->quantized) ? L->w_exp : (int *)nullptr)   // F16X2: same image / exponent protocol as the single-GPU step
+        if (so) {
+            RED_BUCKET(reduce_opt_kernel, *so);
+            DCLL_LAUNCH_OK("reduce_opt_kernel");
+        } else {
+            RED_BUCKET(reduce_adam_kernel, sc);
+            DCLL_LAUNCH_OK("reduce_adam_kernel");
+        }
+#undef RED_BUCKET
         a->adam_i2h.step += 1;
         if (L->quantized) {
             int rc = sync_kernel_weights(L, st);
@@ -429,19 +463,24 @@ int launch_bucket_adam(const dcll_conv_layer *L, dcll_train_args *a, const float
         }
     }
     if (L->output_layer) {
+        OptScalars buf;
+        const OptScalars *sr = next_opt_scalars(a->adam_out, opt ? opt + 1 : nullptr, &buf);
         AdamScalars so = adam_scalars(a->adam_out, a->adam_out.step + 1);
         const float *gwout = bucket + n_tot, *gbout = gwout + (size_t)L->K * g.F;
         ProfScope ps(KC_ADAM, 1, st);
-        int rc = launch_adam_flat(L->wout, gwout, a->adam_out.m_w, a->adam_out.v_w, (size_t)L->K * g.F, so, st);
+        const dcll_adam &o = a->adam_out;
+        int rc = sr ? launch_opt_flat(L->wout, gwout, o.m_w, o.v_w, (size_t)L->K * g.F, *sr, st)
+                    : launch_adam_flat(L->wout, gwout, o.m_w, o.v_w, (size_t)L->K * g.F, so, st);
         if (rc != DCLL_OK) return rc;
-        rc = launch_adam_flat(L->bout, gbout, a->adam_out.m_b, a->adam_out.v_b, (size_t)L->K, so, st);
+        rc = sr ? launch_opt_flat(L->bout, gbout, o.m_b, o.v_b, (size_t)L->K, *sr, st)
+                : launch_adam_flat(L->bout, gbout, o.m_b, o.v_b, (size_t)L->K, so, st);
         if (rc != DCLL_OK) return rc;
         a->adam_out.step += 1;
     }
     return DCLL_OK;
 }
 
-int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st) {
+int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st, const OptScalars *so) {
     Geo g = geo_of(L);
     WsLayout ws = ws_layout(L);
     WgP p;
@@ -461,11 +500,19 @@ int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st) 
         dcll_adam &o = a->adam_i2h;
         ProfScope ps(KC_ADAM, 0, st);
         const int blk = (int)(wgrad_tc2_partial_floats() / 148);
-        launch_k(reduce_adam_rp_kernel, ceil_div(p.n_tot, 64), 256, 0, st, p.partial, nA, nB, blk, blk - L->Cout, p.n_tot, p.nW, L->Cout,
-                 g.CoutPad, L->Cin * L->KH * L->KW, L->weight, L->weight_t, L->bias, o.m_w, o.v_w, o.m_b, o.v_b, a->grad_w, a->grad_b,
-                 a->apply_update, sc, L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma), L->Cin,
-                 L->KH * L->KW, L->KW, (prec_f16(L) && !L->quantized) ? L->w_exp : nullptr);
-        DCLL_LAUNCH_OK("reduce_adam_rp_kernel");
+#define RED_RP(KERN, SC)                                                                                                              \
+    launch_k(KERN, ceil_div(p.n_tot, 64), 256, 0, st, p.partial, nA, nB, blk, blk - L->Cout, p.n_tot, p.nW, L->Cout, g.CoutPad,         \
+             L->Cin * L->KH * L->KW, L->weight, L->weight_t, L->bias, o.m_w, o.v_w, o.m_b, o.v_b, a->grad_w, a->grad_b, a->apply_update, \
+             SC, L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma), L->Cin, L->KH * L->KW, L->KW,              \
+             (prec_f16(L) && !L->quantized) ? L->w_exp : nullptr)
+        if (so) {
+            RED_RP(reduce_opt_rp_kernel, *so);
+            DCLL_LAUNCH_OK("reduce_opt_rp_kernel");
+        } else {
+            RED_RP(reduce_adam_rp_kernel, sc);
+            DCLL_LAUNCH_OK("reduce_adam_rp_kernel");
+        }
+#undef RED_RP
         if (a->apply_update && L->quantized) return sync_kernel_weights(L, st);
         return DCLL_OK;
     }
@@ -486,13 +533,18 @@ int launch_wgrad(const dcll_conv_layer *L, dcll_train_args *a, cudaStream_t st) 
     AdamScalars sc = adam_scalars(a->adam_i2h, a->adam_i2h.step + 1);
     dcll_adam &o = a->adam_i2h;
     ProfScope ps(KC_ADAM, 0, st);
-    launch_k(reduce_adam_kernel, ceil_div(p.n_tot, 64), 256, 0, st, p.partial, p.S, p.n_tot, p.nW, L->Cout, g.CoutPad,
-                                                               L->Cin * L->KH * L->KW, L->weight, L->weight_t, L->bias,
-                                                               o.m_w, o.v_w, o.m_b, o.v_b, a->grad_w, a->grad_b,
-                                                               a->apply_update, sc,
-                                                               L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma),
-                                                               L->Cin, L->KH * L->KW, L->KW, (int *)nullptr);
-    DCLL_LAUNCH_OK("reduce_adam_kernel");
+#define RED(KERN, SC)                                                                                                           \
+    launch_k(KERN, ceil_div(p.n_tot, 64), 256, 0, st, p.partial, p.S, p.n_tot, p.nW, L->Cout, g.CoutPad, L->Cin * L->KH * L->KW,  \
+             L->weight, L->weight_t, L->bias, o.m_w, o.v_w, o.m_b, o.v_b, a->grad_w, a->grad_b, a->apply_update, SC,                \
+             L->quantized ? nullptr : reinterpret_cast<__nv_bfloat16 *>(L->weight_mma), L->Cin, L->KH * L->KW, L->KW, (int *)nullptr)
+    if (so) {
+        RED(reduce_opt_kernel, *so);
+        DCLL_LAUNCH_OK("reduce_opt_kernel");
+    } else {
+        RED(reduce_adam_kernel, sc);
+        DCLL_LAUNCH_OK("reduce_adam_kernel");
+    }
+#undef RED
     // reduce_adam_kernel refreshed weight_t and the tensor-core split itself; only the quantised image needs a pass
     if (a->apply_update && L->quantized) return sync_kernel_weights(L, st);
     return DCLL_OK;

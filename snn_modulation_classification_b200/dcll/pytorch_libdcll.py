@@ -902,6 +902,76 @@ def _store_steps(states, step):
         st['step'] = torch.tensor(float(step), dtype=torch.float32)
 
 
+# optimizers the fused kernels apply (with the single-param-group, non-maximize, non-capturable, non-differentiable options
+# _device_optim checks); any other optimizer takes torch's optimizer.step() in the per-step API
+DEVICE_OPTIMIZERS = ('Adam', 'AdamW', 'Adamax', 'NAdam', 'RAdam')
+
+
+def _device_optim(opt):
+    """The update rule (_lib.OPT_ADAMW / OPT_ADAMAX / OPT_NADAM / OPT_RADAM) the fused kernels apply for `opt`, or None: exact
+    torch.optim.AdamW (or Adam(decoupled_weight_decay=True)) without amsgrad, Adamax, NAdam or RAdam, with one param group,
+    maximize, capturable and differentiable off and a float lr.  Plain Adam is _is_plain_adam's (None here)."""
+    if len(opt.param_groups) != 1:
+        return None
+    g = opt.param_groups[0]
+    if g.get('maximize') or g.get('capturable') or g.get('differentiable') or type(g.get('lr')) is not float:
+        return None
+    t = type(opt)
+    if t is optim.AdamW or (t is optim.Adam and g.get('decoupled_weight_decay')):
+        return None if g.get('amsgrad') else _lib.OPT_ADAMW
+    return {optim.Adamax: _lib.OPT_ADAMAX, optim.NAdam: _lib.OPT_NADAM, optim.RAdam: _lib.OPT_RADAM}.get(t)
+
+
+def _optim_state(opt, p, kind):
+    """optimizer.state[p] exactly as the torch class of rule `kind` lazily creates it, so state_dicts interchange."""
+    st = opt.state[p]
+    if len(st) == 0:
+        st['step'] = torch.tensor(0.0, dtype=torch.float32)
+        if kind == _lib.OPT_NADAM:
+            st['mu_product'] = torch.tensor(1.0, dtype=torch.float32)
+        st['exp_avg'] = torch.zeros_like(p, memory_format=torch.preserve_format)
+        st['exp_inf' if kind == _lib.OPT_ADAMAX else 'exp_avg_sq'] = torch.zeros_like(p, memory_format=torch.preserve_format)
+    return st
+
+
+def _fill_optim(adam, rule, opt, pw, pb):
+    """dcll_adam + dcll_optim of a device optimizer (plain Adam: rule.kind = OPT_ADAM and _fill_adam); returns the states of
+    the weight and the bias, which _store_optim updates after the call."""
+    kind = _lib.OPT_ADAM if _is_plain_adam(opt) else _device_optim(opt)
+    rule.kind = kind
+    if kind == _lib.OPT_ADAM:
+        return _fill_adam(adam, opt, pw, pb)
+    g = opt.param_groups[0]
+    adam.lr, (adam.beta1, adam.beta2) = float(g['lr']), (float(g['betas'][0]), float(g['betas'][1]))
+    adam.eps, adam.weight_decay = float(g['eps']), float(g['weight_decay'])
+    sw, sb = _optim_state(opt, pw, kind), _optim_state(opt, pb, kind)
+    adam.step = int(sw['step'])
+    v = 'exp_inf' if kind == _lib.OPT_ADAMAX else 'exp_avg_sq'
+    adam.m_w, adam.v_w = _lib.ptr(sw['exp_avg']), _lib.ptr(sw[v])
+    adam.m_b, adam.v_b = _lib.ptr(sb['exp_avg']), _lib.ptr(sb[v])
+    rule.decoupled_wd = 1 if g.get('decoupled_weight_decay') else 0
+    rule.momentum_decay = float(g.get('momentum_decay', 0.0))
+    rule.mu_product = float(sw['mu_product']) if kind == _lib.OPT_NADAM else 1.0
+    return sw, sb
+
+
+def _store_optim(states, adam, rule):
+    _store_steps(states, adam.step)
+    if rule.kind == _lib.OPT_NADAM:
+        for st in states:
+            st['mu_product'] = torch.tensor(rule.mu_product, dtype=torch.float32)
+
+
+def _on_device(*opts):
+    """True when every optimizer is one the fused kernels apply (plain Adam or a _device_optim rule)."""
+    return all(_is_plain_adam(o) or _device_optim(o) is not None for o in opts)
+
+
+def _optims_of(s):
+    lay = s.dclllayer
+    return (s.optimizer, s.optimizer2) if lay.output_layer else (s.optimizer,)
+
+
 # ------------------------------------------------------------------------------------------------
 # DCLLBase / DCLLClassification  (ref:615-749)
 # ------------------------------------------------------------------------------------------------
@@ -994,9 +1064,16 @@ class DCLLBase(nn.Module):
             args.loss_out = _lib.ptr(loss_t)
         fused = do_train and _is_plain_adam(self.optimizer) and \
             (not lay.output_layer or _is_plain_adam(self.optimizer2))
+        # AdamW / Adamax / NAdam / RAdam (and plain Adam beside them) go through the _opt entry point
+        rules = (_lib.Optim * 2)() if do_train and not fused and _on_device(*_optims_of(self)) else None
         i2h = lay.i2h
         states = []
-        if fused:
+        if rules is not None:
+            args.apply_update = 1
+            states.append(_fill_optim(args.adam_i2h, rules[0], self.optimizer, i2h.weight, i2h.bias))
+            if lay.output_layer:
+                states.append(_fill_optim(args.adam_out, rules[1], self.optimizer2, lay.output_.weight, lay.output_.bias))
+        elif fused:
             args.apply_update = 1
             states.append(_fill_adam(args.adam_i2h, self.optimizer, i2h.weight, i2h.bias))
             if lay.output_layer:
@@ -1010,15 +1087,22 @@ class DCLLBase(nn.Module):
             args.grad_w, args.grad_b = _lib.ptr(i2h.weight.grad), _lib.ptr(i2h.bias.grad)
             if lay.output_layer:
                 args.grad_wout, args.grad_bout = _lib.ptr(lay.output_.weight.grad), _lib.ptr(lay.output_.bias.grad)
-        _lib.check(_lib.lib.dcll_conv_step_bwd_update(ctypes.byref(desc), ctypes.byref(args), _lib.current_stream()))
-        if fused:
-            _store_steps(states[0], args.adam_i2h.step)
+        if rules is not None:
+            _lib.check(_lib.lib.dcll_conv_step_bwd_update_opt(ctypes.byref(desc), ctypes.byref(args), rules,
+                                                              _lib.current_stream()))
+            _store_optim(states[0], args.adam_i2h, rules[0])
             if lay.output_layer:
-                _store_steps(states[1], args.adam_out.step)
-        elif do_train:
-            self.optimizer.step()                                       # ref:712
-            if lay.output_layer:
-                self.optimizer2.step()                                  # ref:714
+                _store_optim(states[1], args.adam_out, rules[1])
+        else:
+            _lib.check(_lib.lib.dcll_conv_step_bwd_update(ctypes.byref(desc), ctypes.byref(args), _lib.current_stream()))
+            if fused:
+                _store_steps(states[0], args.adam_i2h.step)
+                if lay.output_layer:
+                    _store_steps(states[1], args.adam_out.step)
+            elif do_train:
+                self.optimizer.step()                                   # ref:712
+                if lay.output_layer:
+                    self.optimizer2.step()                              # ref:714
         del keep
         return loss_t
 
@@ -1050,15 +1134,23 @@ class DCLLBase(nn.Module):
         d.g_o, d.g_u = _lib.ptr(g_o), _lib.ptr(g_u)
         d.grad_w, d.grad_b = _lib.ptr(i2h.weight.grad), _lib.ptr(i2h.bias.grad)
         fused = do_train and _is_plain_adam(self.optimizer)
+        rule = _lib.Optim() if do_train and not fused and _device_optim(self.optimizer) is not None else None
         states = None
-        if fused:
+        if rule is not None:
             args.apply_update = 1
-            states = _fill_adam(args.adam_i2h, self.optimizer, i2h.weight, i2h.bias)
-        _lib.check(_lib.lib.dcll_dense_step_bwd_update(ctypes.byref(d), ctypes.byref(args), _lib.current_stream()))
-        if fused:
-            _store_steps(states, args.adam_i2h.step)
-        elif do_train:
-            self.optimizer.step()
+            states = _fill_optim(args.adam_i2h, rule, self.optimizer, i2h.weight, i2h.bias)
+            _lib.check(_lib.lib.dcll_dense_step_bwd_update_opt(ctypes.byref(d), ctypes.byref(args), ctypes.byref(rule),
+                                                               _lib.current_stream()))
+            _store_optim(states, args.adam_i2h, rule)
+        else:
+            if fused:
+                args.apply_update = 1
+                states = _fill_adam(args.adam_i2h, self.optimizer, i2h.weight, i2h.bias)
+            _lib.check(_lib.lib.dcll_dense_step_bwd_update(ctypes.byref(d), ctypes.byref(args), _lib.current_stream()))
+            if fused:
+                _store_steps(states, args.adam_i2h.step)
+            elif do_train:
+                self.optimizer.step()
         lay._g_u = g_u
         del keep
         return loss_t

@@ -14,7 +14,8 @@ import yaml
 
 from .. import _lib
 from ..dcll.pytorch_libdcll import (NATIVE_LOSSES, Conv2dDCLLlayer, DCLLClassification, SpikeCells, _as_cuda_f32,
-                                    _fill_adam, _is_plain_adam, _loss_kind, _store_steps, device)
+                                    _fill_adam, _is_plain_adam, _loss_kind, _store_steps, device,
+                                    DEVICE_OPTIMIZERS, _fill_optim, _on_device, _optims_of, _store_optim)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -180,22 +181,18 @@ class ConvNetwork(torch.nn.Module):
         Layers, Trains = _lib.ConvLayer * n, _lib.TrainArgs * n
         layers, trains = Layers(), Trains()
         olds, states = [], []
+        rules = self._window_rules('learn_window', 'use learn() per timestep') if train else None
         for i, s in enumerate(self.dcll_slices):
             old, _ = s.dclllayer._fill_desc(layers[i], batch, x_mode if i == 0 else _lib.X_DENSE, win['outs'][i])
             olds.append(old)
             if train:
                 lay = s.dclllayer
-                if not (_is_plain_adam(s.optimizer) and (not lay.output_layer or _is_plain_adam(s.optimizer2))):
-                    raise NotImplementedError('learn_window needs torch.optim.Adam slices; use learn() per timestep')
                 kind = _loss_kind(s.crit)
                 if kind == _lib.LOSS_EXTERNAL:
                     raise NotImplementedError('learn_window implements %s with default arguments; use learn()'
                                               % ', '.join(NATIVE_LOSSES))
                 trains[i].loss_kind, trains[i].apply_update = kind, 1
-                st = [_fill_adam(trains[i].adam_i2h, s.optimizer, lay.i2h.weight, lay.i2h.bias)]
-                if lay.output_layer:
-                    st.append(_fill_adam(trains[i].adam_out, s.optimizer2, lay.output_.weight, lay.output_.bias))
-                states.append(st)
+                states.append(self._fill_slice(i, trains[i], rules))
         target, t_stride = None, 0
         if labels is not None:
             target = _as_cuda_f32(labels)
@@ -219,9 +216,14 @@ class ConvNetwork(torch.nn.Module):
         collect = any(getattr(s, 'collect_stats', False) for s in self.dcll_slices)
         hist_cap = T // 20 + 1
         hist = torch.zeros((n, hist_cap, 19), dtype=torch.int32, device=x_t.device) if collect else None
-        _lib.check(_lib.lib.dcll_net_window_stats(layers, trains if train else None, n, _lib.ptr(x_t), _lib.ptr(target),
-                                                  t_stride, T, 1 if train else 0, burnin, iter0, _lib.ptr(clout),
-                                                  _lib.ptr(hist), 20 if collect else 0, hist_cap, _lib.current_stream()))
+        if rules is not None:
+            _lib.check(_lib.lib.dcll_net_window_stats_opt(layers, trains, rules, n, _lib.ptr(x_t), _lib.ptr(target), t_stride, T,
+                                                          1, burnin, iter0, _lib.ptr(clout), _lib.ptr(hist),
+                                                          20 if collect else 0, hist_cap, _lib.current_stream()))
+        else:
+            _lib.check(_lib.lib.dcll_net_window_stats(layers, trains if train else None, n, _lib.ptr(x_t), _lib.ptr(target),
+                                                      t_stride, T, 1 if train else 0, burnin, iter0, _lib.ptr(clout),
+                                                      _lib.ptr(hist), 20 if collect else 0, hist_cap, _lib.current_stream()))
         for i, s in enumerate(self.dcll_slices):
             s.dclllayer.i2h._commit_state(*olds[i], flips=T)
             s.dclllayer._ctx = None
@@ -235,10 +237,44 @@ class ConvNetwork(torch.nn.Module):
                     s.activity_hist.append(hist[i, j].float())
             s.iter += T
             if train:
-                _store_steps(states[i][0], trains[i].adam_i2h.step)
-                if s.dclllayer.output_layer:
-                    _store_steps(states[i][1], trains[i].adam_out.step)
+                self._store_slice(i, trains[i], rules, states[i])
         return clout
+
+    def _window_rules(self, who, hint=''):
+        """None when every slice trains with plain Adam (the Adam entry points); else the dcll_optim array [2 n] of the _opt
+        entry points, when every optimizer is one the device applies.  Raises NotImplementedError otherwise."""
+        opts = [o for s in self.dcll_slices for o in _optims_of(s)]
+        if all(_is_plain_adam(o) for o in opts):
+            return None
+        if not _on_device(*opts):
+            raise NotImplementedError('%s needs %s slices (torch.optim classes, one param group, no amsgrad / maximize / '
+                                      'capturable / differentiable, a float lr)%s'
+                                      % (who, ', '.join(DEVICE_OPTIMIZERS), '; ' + hint if hint else ''))
+        return (_lib.Optim * (2 * self.num_layers))()
+
+    def _fill_slice(self, i, train, rules):
+        """dcll_adam (+ dcll_optim) of slice i's optimizers; returns their states."""
+        s = self.dcll_slices[i]
+        lay = s.dclllayer
+        if rules is None:
+            st = [_fill_adam(train.adam_i2h, s.optimizer, lay.i2h.weight, lay.i2h.bias)]
+            if lay.output_layer:
+                st.append(_fill_adam(train.adam_out, s.optimizer2, lay.output_.weight, lay.output_.bias))
+            return st
+        st = [_fill_optim(train.adam_i2h, rules[2 * i], s.optimizer, lay.i2h.weight, lay.i2h.bias)]
+        if lay.output_layer:
+            st.append(_fill_optim(train.adam_out, rules[2 * i + 1], s.optimizer2, lay.output_.weight, lay.output_.bias))
+        return st
+
+    def _store_slice(self, i, train, rules, states):
+        if rules is None:
+            _store_steps(states[0], train.adam_i2h.step)
+            if self.dcll_slices[i].dclllayer.output_layer:
+                _store_steps(states[1], train.adam_out.step)
+            return
+        _store_optim(states[0], train.adam_i2h, rules[2 * i])
+        if self.dcll_slices[i].dclllayer.output_layer:
+            _store_optim(states[1], train.adam_out, rules[2 * i + 1])
 
     def _dp_handle(self, group, max_ctas):
         """The raw-NCCL communicator of the C driver for `group` (created once: rank 0 draws the unique id, the ranks receive
@@ -286,10 +322,9 @@ class ConvNetwork(torch.nn.Module):
                 logging.warning("Batch size changed from {} to {} since last iteration. Reallocating states."
                                 .format(lay.i2h.state.eps0.shape[0], batch))
                 lay.i2h.init_state(batch, lay.im_dims)
-            if not (_is_plain_adam(s.optimizer) and (not lay.output_layer or _is_plain_adam(s.optimizer2))):
-                raise NotImplementedError('learn_window_dp needs torch.optim.Adam slices')
             if _loss_kind(s.crit) == _lib.LOSS_EXTERNAL:
                 raise NotImplementedError('learn_window_dp implements %s with default arguments' % ', '.join(NATIVE_LOSSES))
+        rules = self._window_rules('learn_window_dp')
         win = self._window_buffers(batch)
         Layers, Trains = _lib.ConvLayer * n, _lib.TrainArgs * n
         layers, trains = Layers(), Trains()
@@ -307,10 +342,7 @@ class ConvNetwork(torch.nn.Module):
             olds.append(old)
             trains[i].loss_kind, trains[i].apply_update = _loss_kind(s.crit), 0
             trains[i].target = _lib.ptr(target)
-            st = [_fill_adam(trains[i].adam_i2h, s.optimizer, lay.i2h.weight, lay.i2h.bias)]
-            if lay.output_layer:
-                st.append(_fill_adam(trains[i].adam_out, s.optimizer2, lay.output_.weight, lay.output_.bias))
-            states.append(st)
+            states.append(self._fill_slice(i, trains[i], rules))
             flat, views = grad_bucket(lay, x_t.device)
             trains[i].grad_w, trains[i].grad_b = _lib.ptr(views[0]), _lib.ptr(views[1])
             if lay.output_layer:
@@ -328,11 +360,15 @@ class ConvNetwork(torch.nn.Module):
             iter0 = (ctypes.c_int32 * n)(*[int(s.iter) for s in self.dcll_slices])
             bptr = (ctypes.c_void_p * n)(*[_lib.ptr(b) for b in buckets])
             bn = (ctypes.c_size_t * n)(*[b.numel() for b in buckets])
-            _lib.check(_lib.lib.dcll_net_window_dp(dp, layers, trains, n, _lib.ptr(x_t), _lib.ptr(target), t_stride, T, burnin,
-                                                   iter0, _lib.ptr(clout), bptr, bn, stream))
+            if rules is not None:
+                _lib.check(_lib.lib.dcll_net_window_dp_opt(dp, layers, trains, rules, n, _lib.ptr(x_t), _lib.ptr(target), t_stride,
+                                                           T, burnin, iter0, _lib.ptr(clout), bptr, bn, stream))
+            else:
+                _lib.check(_lib.lib.dcll_net_window_dp(dp, layers, trains, n, _lib.ptr(x_t), _lib.ptr(target), t_stride, T, burnin,
+                                                       iter0, _lib.ptr(clout), bptr, bn, stream))
             # the side stream's last collective was waited for by the main stream inside the driver: the buckets may be freed
         else:
-            self._learn_window_dp_python(layers, trains, buckets, x_t, target, t_stride, T, clout, group, stream, burnin)
+            self._learn_window_dp_python(layers, trains, buckets, x_t, target, t_stride, T, clout, group, stream, burnin, rules)
         for i, s in enumerate(self.dcll_slices):
             s.dclllayer.i2h._commit_state(*olds[i], flips=T)
             s.dclllayer._ctx = None
@@ -340,16 +376,15 @@ class ConvNetwork(torch.nn.Module):
             if first < T:
                 s.clout.extend(clout[first:, i, :])
             s.iter += T
-            _store_steps(states[i][0], trains[i].adam_i2h.step)
-            if s.dclllayer.output_layer:
-                _store_steps(states[i][1], trains[i].adam_out.step)
+            self._store_slice(i, trains[i], rules, states[i])
         return clout
 
-    def _learn_window_dp_python(self, layers, trains, buckets, x_t, target, t_stride, T, clout, group, stream, burnin):
+    def _learn_window_dp_python(self, layers, trains, buckets, x_t, target, t_stride, T, clout, group, stream, burnin, rules=None):
         """The same schedule issued layer by layer from Python over torch.distributed (any backend)."""
         n = self.num_layers
         pending, needs_apply = [None] * n, [False] * n
         step_bwd, apply = _lib.lib.dcll_conv_step_bwd_update, _lib.lib.dcll_conv_apply_update
+        apply_opt = _lib.lib.dcll_conv_apply_update_opt
         x_stride = x_t[0].numel() * x_t.element_size()
         x_base = x_t.data_ptr()
         iters = [int(s.iter) for s in self.dcll_slices]
@@ -361,7 +396,11 @@ class ConvNetwork(torch.nn.Module):
                 if pending[i] is not None:
                     pending[i].wait()
                     pending[i] = None
-                _lib.check(apply(ctypes.byref(layers[i]), ctypes.byref(trains[i]), stream))
+                if rules is None:
+                    _lib.check(apply(ctypes.byref(layers[i]), ctypes.byref(trains[i]), stream))
+                else:
+                    _lib.check(apply_opt(ctypes.byref(layers[i]), ctypes.byref(trains[i]),
+                                         ctypes.pointer(rules[2 * i]), stream))
                 needs_apply[i] = False
 
         # between two tensor-core layers of equal geometry the next layer's trace update rides in this layer's convolution
