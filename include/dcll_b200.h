@@ -288,7 +288,12 @@ int dcll_net_window_dp_opt(dcll_dp *dp, dcll_conv_layer *layers, dcll_train_args
  * per sample: synaptic traces stay in registers, inter-layer spikes in shared memory, membranes in TMEM (tcgen05, split-bf16).
  * cells: device int32 [Tc][B][2]; pv_out[l]: device float32 [Tc][B][32*256] (sigmoid outputs of layer l, the read-out
  * input).  State (eps0/eps1 of the current half, arp) is read at the start and written back at the end; `cur` is not
- * flipped.  The read-outs then run batched over Tc*B rows with dcll_conv_readout_rows (descriptor with B = Tc*B).      */
+ * flipped.  The read-outs then run batched over Tc*B rows with dcll_conv_readout_rows (descriptor with B = Tc*B).
+ * Operand form of layers 1 and 2, from their descriptors: precision DCLL_PREC_F16X2 runs the f16x2 form of the
+ * per-timestep forward (fp16 traces scaled by 2^a_exp against the fp16 {hi,lo} weight image of w_exp), any other
+ * precision the split-bf16 form; layer 0 runs on the FMA pipe from weight_t in either case.  Quantised layers use the
+ * images dcll_conv_sync_weights left in weight_t / weight_mma.  Layers 1 and 2 of different forms: DCLL_EUNSUPPORTED;
+ * an f16x2 layer without w_exp or with a_exp outside [-100, 100]: DCLL_EINVAL.                                          */
 int dcll_infer_stack16(const dcll_conv_layer *layers, int n_layers, const int32_t *cells, int Tc, float *const *pv_out,
                        void *stream);
 int dcll_conv_readout_rows(const dcll_conv_layer *L, int32_t *clout, void *stream);

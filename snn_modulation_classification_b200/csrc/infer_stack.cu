@@ -10,6 +10,9 @@
 //     from layer to layer live in shared memory as bytes, the membrane accumulators in TMEM;
 //   * layers 1 and 2 run on tcgen05 exactly like conv_fwd_tc.cu (split-bf16, implicit im2col by descriptor shifts,
 //     [W_hi|W_lo] concatenated along N, 12-stage cp.async.bulk weight ring); layer 0 (K = 49) runs on the FMA pipe;
+//   * F16 (DCLL_PREC_F16X2 hidden layers): the operand form of the per-timestep f16x2 forward -- the trace tile is ONE fp16
+//     plane set, fp16(eps1 * 2^a_exp), against the fp16 {hi,lo} image of w * 2^w_exp[0]: one kind::f16 MMA with N = 2C per
+//     K chunk instead of the two bf16 MMAs, the power-of-two scales undone in the epilogue (conv_mma2_kernel's order);
 //   * per timestep only the 8 bytes of the spike cell come in and pv (for the read-outs) goes out.
 //
 // The local read-outs are NOT inside this kernel on purpose: the frozen read-out matrices are 4*K*F bytes per layer
@@ -17,6 +20,7 @@
 // re-stream them every timestep (18 TB/s of L2 traffic across 148 SMs).  Instead pv of the Tc timesteps is written out
 // and readout_fwd_kernel sweeps each read-out matrix ONCE over Tc*B rows (dcll_conv_readout_rows).
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -35,29 +39,39 @@ struct StackP {
     const float *bias[3];
     float alpharp[3], wrp[3];
     float *pv[3];                      // [Tc][B][32*256]
+    int a_exp[3];                      // F16 form, layers 1,2: the trace image holds fp16(eps1 * 2^a_exp)
+    const int *w_exp[3];               // F16 form, layers 1,2: device exponent of the fp16 weight image
 };
 
 namespace st16 {
 constexpr int NT = 512, HW = 16, NPOS = 256, C = 32, KH = 7, KW = 7, NTAPS = 49;
 constexpr int ROWP = HW + KW - 1;                 // 22
 constexpr int PLANE = ROWP * ROWP * 16;           // bytes per channel group of the halo tile
-constexpr int PART = 4 * PLANE, A_BYTES = 2 * PART;
+constexpr int PART = 4 * PLANE;
 constexpr int TAP_BYTES = 2 * 4 * C * 16, NSTAGE = 12;
-constexpr int ACC_COLS = 2 * C, TMEM_COLS = 128;  // 2 M-tiles x [hi*hi+lo*hi | hi*lo]
-constexpr int OFF_RING = A_BYTES;
-constexpr int OFF_SPK = OFF_RING + NSTAGE * TAP_BYTES;        // 2 x [256 pos][32 ch] bytes
-constexpr int OFF_L0 = OFF_SPK + 2 * NPOS * C;                // float [22][24] padded eps1 tile of layer 0
-constexpr int OFF_W0 = OFF_L0 + ROWP * 24 * 4;                // float [49][32]
-constexpr int OFF_COEF = OFF_W0 + NTAPS * C * 4;              // float [2 hidden layers][4][32]
-constexpr int OFF_BIAS = OFF_COEF + 2 * 4 * C * 4;            // float [3][32]
-constexpr int OFF_BAR = OFF_BIAS + 3 * C * 4;
-constexpr int SMEM = OFF_BAR + 256;
+constexpr int ACC_COLS = 2 * C, TMEM_COLS = 128;  // 2 M-tiles x [hi*hi+lo*hi | hi*lo]  (F16: [A*W_hi | A*W_lo])
+template <bool F16>
+struct Smem {
+    static constexpr int A_BYTES = F16 ? PART : 2 * PART;                      // F16: the fp16 part only
+    static constexpr int OFF_RING = A_BYTES;
+    static constexpr int OFF_SPK = OFF_RING + NSTAGE * TAP_BYTES;        // 2 x [256 pos][32 ch] bytes
+    static constexpr int OFF_L0 = OFF_SPK + 2 * NPOS * C;                // float [22][24] padded eps1 tile of layer 0
+    static constexpr int OFF_W0 = OFF_L0 + ROWP * 24 * 4;                // float [49][32]
+    static constexpr int OFF_COEF = OFF_W0 + NTAPS * C * 4;              // float [2 hidden layers][4][32]
+    static constexpr int OFF_BIAS = OFF_COEF + 2 * 4 * C * 4;            // float [3][32]
+    static constexpr int OFF_BAR = OFF_BIAS + 3 * C * 4;
+    static constexpr int SMEM = OFF_BAR + 256;
+};
 }  // namespace st16
 
+template <bool F16>
 __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP p) {
     pdl_entry();
     using namespace st16;
     using namespace tc;
+    using S = Smem<F16>;
+    constexpr int A_BYTES = S::A_BYTES, OFF_RING = S::OFF_RING, OFF_SPK = S::OFF_SPK, OFF_L0 = S::OFF_L0, OFF_W0 = S::OFF_W0,
+                  OFF_COEF = S::OFF_COEF, OFF_BIAS = S::OFF_BIAS, OFF_BAR = S::OFF_BAR;
     extern __shared__ __align__(128) unsigned char smem[];
     unsigned char *sA = smem, *sW = smem + OFF_RING;
     unsigned char *spk[2] = {smem + OFF_SPK, smem + OFF_SPK + NPOS * C};
@@ -114,6 +128,12 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
         }
 
     constexpr uint32_t IDESC_N2 = idesc_bf16(128, 2 * C, false, false), IDESC_N1 = idesc_bf16(128, C, false, false);
+    constexpr uint32_t IDESC_F16 = idesc_f16a(128, 2 * C, false, false);
+    float unscale[2] = {1.f, 1.f};
+    if constexpr (F16) {
+#pragma unroll
+        for (int l = 0; l < 2; ++l) unscale[l] = pow2i(-(p.a_exp[l + 1] + __ldg(p.w_exp[l + 1])));
+    }
     constexpr uint32_t A_HI = desc_hi(ROWP * 16), B_HI = desc_hi(128);
     const uint32_t a_lo_base = desc_lo(smem_u32(sA), PLANE), b_lo_base = desc_lo(smem_u32(sW), 2 * C * 16);
     const uint32_t elected = elect_one();
@@ -194,13 +214,14 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
                 }
             }
             __syncthreads();   // spikes of the previous layer are complete (and layer 0's tile reads are done)
-            // ---- prologue: trace update in registers, bf16 hi/lo split into the A tile interior
+            // ---- prologue: trace update in registers, bf16 hi/lo split (F16: the scaled fp16 value) into the A tile interior
             const float *cf = coef + l * 4 * C;
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
                 const int cg = half + 2 * h;
                 const uint2 xb = *reinterpret_cast<const uint2 *>(spk[l] + pos * C + cg * 8);
                 __align__(16) __nv_bfloat16 hi[8], lo[8];
+                __align__(16) __half hf[8];
 #pragma unroll
                 for (int k = 0; k < 8; ++k) {
                     const int ch = cg * 8 + k;
@@ -208,12 +229,20 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
                     const float n0 = __fadd_rn(__fmul_rn(xin, cf[ch]), __fmul_rn(cf[C + ch], he0[l][h][k]));
                     const float n1 = __fadd_rn(__fmul_rn(cf[2 * C + ch], he1[l][h][k]), __fmul_rn(n0, cf[3 * C + ch]));
                     he0[l][h][k] = n0, he1[l][h][k] = n1;
-                    hi[k] = __float2bfloat16_rn(n1);
-                    lo[k] = __float2bfloat16_rn(n1 - __bfloat162float(hi[k]));
+                    if constexpr (F16) {
+                        hf[k] = __float2half_rn(__fmul_rn(n1, pow2i(p.a_exp[l + 1])));
+                    } else {
+                        hi[k] = __float2bfloat16_rn(n1);
+                        lo[k] = __float2bfloat16_rn(n1 - __bfloat162float(hi[k]));
+                    }
                 }
                 unsigned char *dst = sA + cg * PLANE + ((r + 3) * ROWP + c + 3) * 16;
-                *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(hi);
-                *reinterpret_cast<uint4 *>(dst + PART) = *reinterpret_cast<const uint4 *>(lo);
+                if constexpr (F16) {
+                    *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(hf);
+                } else {
+                    *reinterpret_cast<uint4 *>(dst) = *reinterpret_cast<const uint4 *>(hi);
+                    *reinterpret_cast<uint4 *>(dst + PART) = *reinterpret_cast<const uint4 *>(lo);
+                }
             }
             fence_async_smem();
             __syncthreads();
@@ -234,8 +263,12 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
 #pragma unroll
                             for (int j = 0; j < 2; ++j) {
                                 const uint64_t bd = desc(B_HI, b_tap + ((2 * j * 2 * C * 16) >> 4));
-                                mma_bf16(d, desc(A_HI, a_tap + ((2 * j * PLANE) >> 4)), bd, IDESC_N2, (i | j) != 0);
-                                mma_bf16(d, desc(A_HI, a_tap + ((PART + 2 * j * PLANE) >> 4)), bd, IDESC_N1, 1);
+                                if constexpr (F16) {
+                                    mma_bf16(d, desc(A_HI, a_tap + ((2 * j * PLANE) >> 4)), bd, IDESC_F16, (i | j) != 0);
+                                } else {
+                                    mma_bf16(d, desc(A_HI, a_tap + ((2 * j * PLANE) >> 4)), bd, IDESC_N2, (i | j) != 0);
+                                    mma_bf16(d, desc(A_HI, a_tap + ((PART + 2 * j * PLANE) >> 4)), bd, IDESC_N1, 1);
+                                }
                             }
                         }
                         commit(empty + s);
@@ -283,7 +316,9 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
 #pragma unroll
                     for (int k = 0; k < 16; ++k) {
                         const int co = n0 + k;
-                        float u = __fadd_rn(__fadd_rn(__uint_as_float(v[k]), __uint_as_float(v2[k])), bias_s[(l + 1) * C + co]);
+                        float u = __fadd_rn(__uint_as_float(v[k]), __uint_as_float(v2[k]));
+                        if constexpr (F16) u = __fmul_rn(u, unscale[l]);      // undo the power-of-two operand scales (exact)
+                        u = __fadd_rn(u, bias_s[(l + 1) * C + co]);
                         float a = 0.f;
                         if (arp) {
                             a = __fmul_rn(p.alpharp[l + 1], av[k]);
@@ -325,7 +360,7 @@ __global__ void __launch_bounds__(st16::NT, 1) infer_stack16_kernel(const StackP
     if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-static int stack16_check(const dcll_conv_layer *Ls, int n_layers) {
+static int stack16_check(const dcll_conv_layer *Ls, int n_layers, bool *f16) {
     DCLL_REQUIRE(Ls && n_layers == 3, DCLL_EUNSUPPORTED, "dcll_infer_stack16: needs exactly 3 layers");
     for (int l = 0; l < 3; ++l) {
         const dcll_conv_layer &L = Ls[l];
@@ -333,10 +368,25 @@ static int stack16_check(const dcll_conv_layer *Ls, int n_layers) {
                          L.Cout == 32 && L.Cin == (l == 0 ? 1 : 32) && L.B == Ls[0].B,
                      DCLL_EUNSUPPORTED, "dcll_infer_stack16: layer %d is not a 16x16, 7x7/pad 3, %d->32 channel layer", l, l ? 32 : 1);
         DCLL_REQUIRE(L.coef_mode != DCLL_COEF_ELEMENT, DCLL_EUNSUPPORTED, "dcll_infer_stack16: per-element time constants unsupported");
-        DCLL_REQUIRE(!L.quantized, DCLL_EUNSUPPORTED, "dcll_infer_stack16: quantised weights unsupported");
         DCLL_REQUIRE(L.weight_t && L.bias && L.eps0[L.cur & 1] && L.eps1[L.cur & 1] && (l == 0 || L.weight_mma) && (!(L.wrp > 0.f) || L.arp),
                      DCLL_EINVAL, "dcll_infer_stack16: null tensor in layer %d", l);
     }
+    // operand form of the tensor-core layers 1 and 2: fp16 traces (f16x2) or split-bf16; one kernel instantiation runs both
+    *f16 = Ls[1].precision == DCLL_PREC_F16X2;
+    DCLL_REQUIRE((Ls[2].precision == DCLL_PREC_F16X2) == *f16, DCLL_EUNSUPPORTED,
+                 "dcll_infer_stack16: layers 1 and 2 differ in operand form (one f16x2, one split-bf16)");
+    for (int l = 1; l < 3 && *f16; ++l) {
+        DCLL_REQUIRE(Ls[l].w_exp, DCLL_EINVAL, "dcll_infer_stack16: f16x2 layer %d has no w_exp", l);
+        DCLL_REQUIRE(Ls[l].a_exp >= -100 && Ls[l].a_exp <= 100, DCLL_EINVAL, "dcll_infer_stack16: f16x2 layer %d: a_exp out of range", l);
+    }
+    return DCLL_OK;
+}
+
+template <bool F16>
+static int launch_stack16(const StackP &p, cudaStream_t st) {
+    DCLL_SMEM_ATTR(infer_stack16_kernel<F16>, st16::Smem<F16>::SMEM);
+    launch_k(infer_stack16_kernel<F16>, p.B, st16::NT, st16::Smem<F16>::SMEM, st, p);
+    DCLL_LAUNCH_OK("infer_stack16_kernel");
     return DCLL_OK;
 }
 
@@ -346,7 +396,8 @@ using namespace dcll;
 
 extern "C" __attribute__((visibility("default"))) int dcll_infer_stack16(const dcll_conv_layer *layers, int n_layers, const int32_t *cells,
                                                                          int Tc, float *const *pv_out, void *stream) {
-    int rc = stack16_check(layers, n_layers);
+    bool f16 = false;
+    int rc = stack16_check(layers, n_layers, &f16);
     if (rc != DCLL_OK) return rc;
     DCLL_REQUIRE(cells && pv_out && pv_out[0] && pv_out[1] && pv_out[2] && Tc > 0, DCLL_EINVAL, "dcll_infer_stack16: bad arguments");
     StackP p;
@@ -359,12 +410,10 @@ extern "C" __attribute__((visibility("default"))) int dcll_infer_stack16(const d
         p.alpha[l] = L.alpha, p.alphas[l] = L.alphas, p.tau_m[l] = L.tau_m, p.tau_s[l] = L.tau_s, p.coef_mode[l] = L.coef_mode;
         p.w_mma[l] = reinterpret_cast<const __nv_bfloat16 *>(L.weight_mma);
         p.bias[l] = L.bias, p.alpharp[l] = L.alpharp, p.wrp[l] = L.wrp, p.pv[l] = pv_out[l];
+        p.a_exp[l] = f16 ? L.a_exp : 0, p.w_exp[l] = f16 ? L.w_exp : nullptr;
     }
     p.w0t = layers[0].weight_t;   // [49][32] since CoutPad == 32
-    DCLL_SMEM_ATTR(infer_stack16_kernel, st16::SMEM);
-    launch_k(infer_stack16_kernel, p.B, st16::NT, st16::SMEM, (cudaStream_t)stream, p);
-    DCLL_LAUNCH_OK("infer_stack16_kernel");
-    return DCLL_OK;
+    return f16 ? launch_stack16<true>(p, (cudaStream_t)stream) : launch_stack16<false>(p, (cudaStream_t)stream);
 }
 
 // Read-outs of `rows` rows of pv (rows = Tc*B after dcll_infer_stack16): L->B must be set to `rows`, L->pv / pvoutput / output /

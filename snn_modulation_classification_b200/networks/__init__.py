@@ -54,6 +54,7 @@ def load_network_spec(yaml_path):
 
 
 _DP_HANDLES = {}
+STACK16_F16X2_MAX_BATCH = 4096      # largest batch for which test_window runs dcll_infer_stack16 in 'f16x2'
 
 
 def grad_bucket(lay, dev):
@@ -104,6 +105,9 @@ class ConvNetwork(torch.nn.Module):
                                               optimizer=opt, kwargs_optimizer=layer_opt_param, collect_stats=True,
                                               burnin=burnin))
         self._win = None
+        # the training / inference CLIs' --precision (a mode of the layers, not a parameter: it survives .to() and
+        # load_state_dict); callers whose args carry none keep 'fp32'
+        self.set_precision(getattr(args, 'precision', 'fp32'))
 
     def set_precision(self, mode):
         """'fp32': FP32-exact parity mode (CUDA-core FMA).  'bf16x3': convolutions of the layers with an
@@ -429,7 +433,8 @@ class ConvNetwork(torch.nn.Module):
 
     def test_window(self, x):
         """``for t in range(T): self.test(x[t])`` (test_radio_ml.py:144-145) in one call.  The radio_ml_conv stack on a
-        16x16 plane in 'bf16x3' mode with cell input takes the multi-timestep kernel (state on chip across timesteps)."""
+        16x16 plane in 'bf16x3' or 'f16x2' mode, quantised or not, with cell input takes the multi-timestep kernel (state on
+        chip across timesteps), in the operand form of the per-timestep kernels of that mode."""
         if self._stack16_ok(x):
             return self._run_stack16(x)
         return self._run_window(x, None, False)
@@ -442,9 +447,15 @@ class ConvNetwork(torch.nn.Module):
             lay, i2h = s.dclllayer, s.dclllayer.i2h
             if (tuple(int(v) for v in lay.im_dims) != (16, 16) or i2h.kernel_size != (7, 7) or i2h.padding != (3, 3)
                     or tuple(lay.pooling) != (1, 1) or i2h.out_channels != 32 or i2h.in_channels != (1 if i == 0 else 32)
-                    or i2h.precision != 'bf16x3' or i2h.quantized or i2h.state.eps0.shape[0] != x.cells.shape[1]):
+                    or i2h.precision not in ('bf16x3', 'f16x2') or i2h.state.eps0.shape[0] != x.cells.shape[1]):
                 return False
-        return True
+        # one kernel instantiation runs both 32 -> 32 layers: same operand form
+        mode = self.dcll_slices[1].dclllayer.i2h.precision
+        if mode != self.dcll_slices[2].dclllayer.i2h.precision:
+            return False
+        # f16x2: faster than the per-timestep f16x2 kernels up to B = 4096 (B200, T = 256), slower at B = 65536, where the pv
+        # buffer holds one timestep per launch (DESIGN §4.5); larger batches keep the per-timestep kernels
+        return mode != 'f16x2' or x.cells.shape[1] <= STACK16_F16X2_MAX_BATCH
 
     def _run_stack16(self, x, chunk=None):
         n, cells = 3, x.cells

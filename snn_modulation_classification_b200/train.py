@@ -74,6 +74,9 @@ def parse_args(argv=None):
     p.add_argument('--netscale', type=float, default=1.)
     p.add_argument('--comment', type=str, default='')
     p.add_argument('--output', type=str, default='results')
+    p.add_argument('--precision', type=str, default='fp32', choices=['fp32', 'bf16x3', 'f16x2'],
+                   help="convolution arithmetic (ConvNetwork.set_precision): 'fp32' is FP32-exact, 'bf16x3' and 'f16x2' run "
+                        "the tcgen05 tensor-core kernels where the layer shape has them")
     return p.parse_args(argv)
 
 
